@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--frames F] [--distinct G] [--rgb-scale S] [--e2e-frames E] [--pipeline fused|split]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of F synthetic 1920x1088 High-profile IDR pictures
 (BASELINE.json configs[2]) that are already resident in HBM: ONE launch of the fused kernel kf_recon
@@ -334,6 +335,15 @@ def run_ours(args):
     dev_ms, mean_ms, launches, t_wall0, t_wall1 = timed_resident(F, scale, split)
     wall_ms = (t_wall1 - t_wall0) * 1e3
     clocks = sampler.result(t_wall0, t_wall1)
+    dump = None
+    if args.dump_outputs and rank == 0:
+        # the RGB24 pictures the last timed step left in HBM, before the other pipeline overwrites them; F full pictures
+        # are gigabytes, so a fixed seeded sample: every eighth row (seeded choice) of eight pictures (seeded choice)
+        rng = np.random.default_rng(0xC0FFEE)
+        dump_slots = np.sort(rng.choice(F, min(F, 8), replace=False))
+        dump_rows = np.sort(rng.choice(H // scale, max(1, H // scale // 8), replace=False))
+        dump = {"rgb": np.stack([ctx.download_rgb(int(s), scale)[dump_rows] for s in dump_slots]).astype(np.float32),
+                "rgb_slots": dump_slots.astype(np.float64), "rgb_rows": dump_rows.astype(np.float64)}
     # what was timed produced the right pictures: a source slot, a clone in the middle, one of the last slots
     for s in sorted({probe[-1], (F // 2) // G * G + probe[0] if F >= 2 * G else probe[0], (F - 1) // G * G + probe[0] if F > G else probe[0]}):
         if s < F:
@@ -627,6 +637,10 @@ def run_ours(args):
             except Exception as e:
                 line["cpu_baseline"] = {"value": None, "unit": UNIT, "cores": 0, "kind": "reference", "sample": f"unavailable: {e}"}
         print(json.dumps(line), flush=True)
+    if dump is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), a)
     ctx.close()
     if world > 1:
         dist.barrier()
@@ -651,7 +665,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs3", dest="configs3", action="store_false", help="skip the configs[3] block (8000 pictures, 1/4-size RGB)")
     ap.add_argument("--pipeline", default="fused", choices=["fused", "split"], help="fused kernel (default) or round 1's three kernels")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write a seeded sample of the RGB24 output of the last step as float32 DIR/rgb.npy "
+                         "(rank 0; picture slots and rows in DIR/rgb_slots.npy, DIR/rgb_rows.npy); "
+                         "--impl reference writes nothing")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

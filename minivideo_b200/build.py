@@ -31,6 +31,15 @@ NVCC_FLAGS = [
 ]
 
 
+def _reference_has(rel: str) -> bool:
+    """Whether the reference tree holds `rel`; a tree this user may not read counts as absent."""
+    p = REFERENCE / rel
+    try:
+        return p.exists() and os.access(p, os.R_OK)
+    except OSError:
+        return False
+
+
 def _stale(target: Path, sources: list[Path]) -> bool:
     if not target.exists():
         return True
@@ -108,7 +117,7 @@ def build_oracle(force: bool = False) -> Path:
 def build_reference(force: bool = False) -> Path | None:
     """Compile the unmodified reference (only where its tree is mounted)."""
     out = ROOT / "oracle" / "_ref" / "ref_decode"
-    if not (REFERENCE / "minivideo" / "src").is_dir():
+    if not _reference_has("minivideo/src"):
         return out if out.exists() else None
     if force or _stale(out, [ROOT / "oracle" / "ref_driver.c", ROOT / "oracle" / "ref_png.c", ROOT / "oracle" / "Makefile"]):
         _run(["make", "-C", str(ROOT / "oracle"), "ref", f"REF={REFERENCE}", "-j8"])
@@ -119,7 +128,7 @@ def build_shim_cli(force: bool = False) -> Path | None:
     """The reference's own mini_thumbnailer main.cpp linked against libminivideo_b200.so (only where the
     reference tree is mounted; the binary lives in oracle/_ref and travels to the GPU box)."""
     out = ROOT / "oracle" / "_ref" / "mini_thumbnailer_b200"
-    if not (REFERENCE / "mini_thumbnailer" / "src" / "main.cpp").exists():
+    if not _reference_has("mini_thumbnailer/src/main.cpp"):
         return out if out.exists() else None
     if force or _stale(out, [PKG / "libminivideo_b200.so", ROOT / "oracle" / "Makefile"]):
         _run(["make", "-C", str(ROOT / "oracle"), "shimcli", f"REF={REFERENCE}"])

@@ -1,8 +1,10 @@
 """Shared helpers for the tests."""
 from __future__ import annotations
 
+import functools
 import hashlib
 import json
+import os
 import struct
 import zlib
 from pathlib import Path
@@ -33,6 +35,46 @@ def large_digests():
 
 def sha(a) -> str:
     return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+def digest(b: bytes) -> str:
+    return hashlib.sha256(b).hexdigest()
+
+
+# Expected results of the tests that compare with the reference's binaries, for machines without oracle/_ref.  Where
+# they come from: the reference's sources were not available when the file was made, so it was recorded with
+# MVG_RECORD_REFERENCE from this project's own writers, mv_thumbnailer, front end and CPU oracle standing in for the
+# reference binaries, at the code whose GPU suite last passed against the built reference.  Until it is re-recorded
+# from the reference itself it therefore pins this project's results; every run where oracle/_ref is built checks
+# each stored entry against the reference and fails on a difference.
+REFERENCE_OUTPUTS = GOLDEN / "reference_outputs.json"
+
+
+def reference_output(key: str, live, available: bool):
+    """The result for one test case of the reference's binaries (oracle/_ref, built by oracle/Makefile from the
+    reference's sources, which are not part of this repository), as JSON data: SHA-256 digests of files and arrays,
+    picture indices.  Where they are built, live() runs them and the result must equal the entry stored in
+    golden/reference_outputs.json; elsewhere the stored entry stands in (see REFERENCE_OUTPUTS for its source).  With
+    MVG_RECORD_REFERENCE=FILE every live result is collected into FILE instead of being checked: run the suite so
+    where oracle/_ref is built, and copy FILE over golden/reference_outputs.json to re-record it."""
+    recorded = _recorded_reference_outputs()
+    if available:
+        out = live()
+        rec_path = os.environ.get("MVG_RECORD_REFERENCE")
+        if rec_path:
+            rec = json.loads(Path(rec_path).read_text()) if Path(rec_path).exists() else {}
+            rec[key] = out
+            Path(rec_path).write_text(json.dumps(rec, indent=1, sort_keys=True) + "\n")
+        else:
+            assert key in recorded and recorded[key] == out, f"golden/reference_outputs.json differs from the reference for {key!r}"
+        return out
+    assert key in recorded, f"no stored reference output for {key!r} (tests/golden/reference_outputs.json)"
+    return recorded[key]
+
+
+@functools.lru_cache(maxsize=None)
+def _recorded_reference_outputs() -> dict:
+    return json.loads(REFERENCE_OUTPUTS.read_text())
 
 
 def oracle_sps_from_tables(soa, ls4, ls8):

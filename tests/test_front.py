@@ -84,30 +84,34 @@ def _interleaved_stream(n, seed=9):
     return out + b"\x00" * 64
 
 
-@pytest.mark.skipif(not ref.available(), reason="oracle/_ref not built")
 @pytest.mark.parametrize("mode,flag", [(1, "ordered"), (2, "distributed")])
 @pytest.mark.parametrize("n_total,n_want", [(20, 5), (60, 7), (31, 4)])
 def test_idr_selection_matches_the_reference_filter(mode, flag, n_total, n_want, tmp_path):
     """mvf_select_idr() vs idr_filtering() (demuxer/filter.c): run the reference CLI with -e ordered /
     distributed and identify which pictures it exported."""
     import subprocess
+    from helpers import reference_output
     from minivideo_b200 import front
     stream = _interleaved_stream(n_total)
     st = front.Stream(stream)
     assert st.n_idr == n_total
-    every = ref.decode(stream, n_total, 64, 48)["yuv"]
-    (tmp_path / "in.264").write_bytes(stream)
-    subprocess.run([str(ref.MINI_THUMBNAILER), "-i", "in.264", "-f", "yuv420", "-n", str(n_want), "-e", flag],
-                   cwd=tmp_path, capture_output=True)
-    got = []
-    for i in range(n_want):
-        f = tmp_path / f"in_{i}.yuv"
-        if not f.exists():
-            break
-        pic = np.fromfile(f, np.uint8)
-        hits = [k for k in range(n_total) if np.array_equal(every[k], pic)]
-        assert hits, "reference exported a picture that is not in the stream"
-        got.append(hits[0])
+
+    def live():
+        every = ref.decode(stream, n_total, 64, 48)["yuv"]
+        (tmp_path / "in.264").write_bytes(stream)
+        subprocess.run([str(ref.MINI_THUMBNAILER), "-i", "in.264", "-f", "yuv420", "-n", str(n_want), "-e", flag],
+                       cwd=tmp_path, capture_output=True)
+        exported = []
+        for i in range(n_want):
+            f = tmp_path / f"in_{i}.yuv"
+            if not f.exists():
+                break
+            pic = np.fromfile(f, np.uint8)
+            hits = [k for k in range(n_total) if np.array_equal(every[k], pic)]
+            assert hits, "reference exported a picture that is not in the stream"
+            exported.append(hits[0])
+        return exported
+    got = reference_output(f"mini_thumbnailer -e {flag} -n {n_want} of {n_total}", live, ref.available())
     mine = st.select_idr(n_want, mode).tolist()
     assert mine[:len(got)] == got and len(mine) >= len(got)
     assert len(got) >= n_want - 1            # the reference may lose the last one (index one past the end)

@@ -9,6 +9,7 @@ from pathlib import Path
 import numpy as np
 import pytest
 
+from helpers import digest, reference_output
 from helpers import png_decode as decode
 
 ROOT = Path(__file__).resolve().parent.parent
@@ -67,12 +68,11 @@ def pictures():
     yield "few colours", rng.integers(0, 4, (120, 200, 3)) * 60
 
 
-@pytest.mark.skipif(not REF_PNG.exists(), reason="oracle/_ref/ref_png not built")
 @pytest.mark.parametrize("name,img", list(pictures()), ids=[n for n, _ in pictures()])
 def test_png_bytes_equal_the_reference_writer(lib, name, img):
     img = np.asarray(img, np.uint8)
-    got, want = encode(lib, img), reference(img)
-    assert got == want
+    want = reference_output(f"ref_png {name}", lambda: digest(reference(img)), REF_PNG.exists())
+    assert digest(encode(lib, img)) == want
 
 
 @pytest.mark.parametrize("name,img", [p for p in pictures() if p[0] in ("1x1", "noise", "blocks+noise", "repeat")],
@@ -90,12 +90,12 @@ def test_png_rejects_bad_arguments(lib):
     assert not lib.mvt_png_encode(buf.ctypes.data, 4, -1, C.byref(n))
 
 
-@pytest.mark.skipif(not REF_PNG.exists(), reason="oracle/_ref/ref_png not built")
 def test_png_random_small_images_equal_the_reference_writer(lib):
     """Sizes 1..40 and contents from flat to noise, with repeats at random distances: the corner cases of the
     filter choice (ties, first row) and of the match finder (matches at the very end, overlapping matches,
     the lazy step) show up in small pictures far more often than in large ones."""
     rng = np.random.default_rng(77)
+    cases = []
     for k in range(60):
         w, h = int(rng.integers(1, 41)), int(rng.integers(1, 41))
         kind = k % 4
@@ -109,5 +109,7 @@ def test_png_random_small_images_equal_the_reference_writer(lib):
         else:
             yy, xx = np.mgrid[0:h, 0:w]
             img = np.stack([xx * 7 + yy, xx + yy * 5, (xx * yy) % 17], -1) + rng.integers(0, 2, (h, w, 3))
-        img = np.asarray(img & 255, np.uint8)
-        assert encode(lib, img) == reference(img), (k, w, h, kind)
+        cases.append((k, w, h, kind, np.asarray(img & 255, np.uint8)))
+    want = reference_output("ref_png random_small", lambda: [digest(reference(c[-1])) for c in cases], REF_PNG.exists())
+    for (k, w, h, kind, img), d in zip(cases, want, strict=True):
+        assert digest(encode(lib, img)) == d, (k, w, h, kind)

@@ -1,5 +1,7 @@
 """mv_thumbnailer (bitstream -> front end -> C ABI -> picture files) against the files the unmodified
-reference CLI (oracle/_ref/mini_thumbnailer) writes for the same stream and arguments: byte for byte."""
+reference CLI (oracle/_ref/mini_thumbnailer) writes for the same stream and arguments: byte for byte (SHA-256), live
+where oracle/_ref is built, elsewhere against the digests stored in tests/golden/reference_outputs.json (where they
+come from: tests/helpers.py, REFERENCE_OUTPUTS)."""
 import os
 import subprocess
 import tempfile
@@ -8,6 +10,7 @@ from pathlib import Path
 import numpy as np
 import pytest
 
+from helpers import digest, reference_output
 from oracle import ref
 
 ROOT = Path(__file__).resolve().parent.parent
@@ -64,23 +67,36 @@ def test_reference_cli_linked_against_the_drop_in_library(cli, fmt, n, mode):
     if not (SHIM_CLI.exists() and ref.MINI_THUMBNAILER.exists()):
         pytest.skip("reference CLI builds are not present")
     stream, _ = synth.generate(9, "cif", seed=905)
-    want, got = _run_both(stream, ["-f", fmt, "-n", str(n), "-e", mode], exes=((ref.MINI_THUMBNAILER, []), (SHIM_CLI, [])))
+    args = ["-f", fmt, "-n", str(n), "-e", mode]
+    (want, r1), (got, r2) = _run(ref.MINI_THUMBNAILER, stream, args), _run(SHIM_CLI, stream, args)
+    assert r1.returncode == 0 and r2.returncode == 0, (r1.stderr[-1500:], r2.stderr[-1500:])
     assert sorted(want) == sorted(got) and len(want) == n
     for name in want:
         assert want[name] == got[name], name
 
 
-def _run_both(stream: bytes, args: list[str], ref_may_crash: bool = False, exes=None):
-    """Run both CLIs in separate scratch directories on the same stream; return {file name: bytes} each."""
-    out = []
-    for exe, extra in (exes or ((ref.MINI_THUMBNAILER, []), (MV, ["-o", "."]))):
-        with tempfile.TemporaryDirectory(dir="/dev/shm" if os.path.isdir("/dev/shm") else None) as d:
-            (Path(d) / "in.264").write_bytes(stream)
-            r = subprocess.run([str(exe), "-i", str(Path(d) / "in.264")] + args + extra, capture_output=True, text=True, cwd=d)
-            if not (ref_may_crash and exe == ref.MINI_THUMBNAILER):
-                assert r.returncode == 0, (exe, r.stdout[-1500:], r.stderr[-1500:])
-            out.append({p.name: p.read_bytes() for p in Path(d).iterdir() if p.name != "in.264"})
-    return out
+def _run(exe, stream: bytes, args: list[str]):
+    """Run one CLI in a scratch directory on the stream; return ({file name: bytes}, the finished process)."""
+    with tempfile.TemporaryDirectory(dir="/dev/shm" if os.path.isdir("/dev/shm") else None) as d:
+        (Path(d) / "in.264").write_bytes(stream)
+        r = subprocess.run([str(exe), "-i", str(Path(d) / "in.264")] + args, capture_output=True, text=True, cwd=d)
+        return {p.name: p.read_bytes() for p in Path(d).iterdir() if p.name != "in.264"}, r
+
+
+def _reference_files(stream: bytes, args: list[str], may_crash: bool = False, keep=lambda data: True):
+    """{file name: SHA-256} of the files the reference CLI writes, core dumps left out; a file `keep` rejects maps to None."""
+    def live():
+        files, r = _run(ref.MINI_THUMBNAILER, stream, args)
+        assert may_crash or r.returncode == 0, (r.stdout[-1500:], r.stderr[-1500:])
+        return {k: digest(v) if keep(v) else None for k, v in files.items() if not k.startswith("core")}
+    return reference_output(f"mini_thumbnailer {digest(stream)[:16]} {' '.join(args)}", live, ref.MINI_THUMBNAILER.exists())
+
+
+def _run_both(stream: bytes, args: list[str], ref_may_crash: bool = False):
+    """The files the reference CLI and mv_thumbnailer write for the same stream and arguments, {file name: SHA-256} each."""
+    files, r = _run(MV, stream, args + ["-o", "."])
+    assert r.returncode == 0, (r.stdout[-1500:], r.stderr[-1500:])
+    return _reference_files(stream, args, ref_may_crash), {k: digest(v) for k, v in files.items()}
 
 
 @pytest.mark.gpu
@@ -88,14 +104,11 @@ def _run_both(stream: bytes, args: list[str], ref_may_crash: bool = False, exes=
 @pytest.mark.parametrize("mode,n", [("unfiltered", 1), ("unfiltered", 5), ("ordered", 4), ("distributed", 4)])
 def test_cli_files_equal_the_reference_cli(cli, fmt, mode, n):
     from minivideo_b200 import synth
-    if not ref.MINI_THUMBNAILER.exists():
-        pytest.skip("reference CLI not built")
     stream, _ = synth.generate(12, "cif", seed=901)
     # 'distributed' indexes one past its candidate list in the reference (demuxer/filter.c:179-186) and
     # can abort after writing some of the pictures: compare what it did write
     crashy = mode == "distributed"
     want, got = _run_both(stream, ["-f", fmt, "-n", str(n), "-e", mode], ref_may_crash=crashy)
-    want = {k: v for k, v in want.items() if not k.startswith("core")}
     if crashy:
         assert set(want) <= set(got) and len(want) >= n - 1
         want.pop(sorted(want)[-1])          # the last file may be cut short by the abort
@@ -111,8 +124,6 @@ def test_cli_default_format_and_jpg_are_written_as_png_like_the_reference_build(
     """mini_thumbnailer defaults to 'jpg' (main.cpp:56); the reference build without libjpeg writes PNG files for
     it (export.c:652-657) through its vendored stb writer."""
     from minivideo_b200 import synth
-    if not ref.MINI_THUMBNAILER.exists():
-        pytest.skip("reference CLI not built")
     stream, _ = synth.generate(3, width_mbs=20, height_mbs=12, profile_idc=100, transform8x8=1, scaling_lists=1, seed=911)
     want, got = _run_both(stream, args + ["-n", "3"])
     assert sorted(want) == sorted(got) == ["in_0.png", "in_1.png", "in_2.png"]
@@ -122,8 +133,6 @@ def test_cli_default_format_and_jpg_are_written_as_png_like_the_reference_build(
 @pytest.mark.gpu
 def test_cli_high_profile_stream_and_small_batches(cli):
     from minivideo_b200 import synth
-    if not ref.MINI_THUMBNAILER.exists():
-        pytest.skip("reference CLI not built")
     stream, _ = synth.generate(7, width_mbs=20, height_mbs=12, profile_idc=100, transform8x8=1, scaling_lists=1,
                                cb_qp_offset=3, cr_qp_offset=-1, seed=902)
     want, _ = _run_both(stream, ["-f", "bmp", "-n", "7"])
@@ -177,13 +186,14 @@ def test_cli_2160p_distributed_extraction(cli):
     """BASELINE.json configs[4]: a 3840x2160 High-profile stream in 'distributed' extraction mode, through the
     CLI, against the files of the reference CLI (which may abort after writing them, see above)."""
     from minivideo_b200 import synth
-    if not ref.MINI_THUMBNAILER.exists():
-        pytest.skip("reference CLI not built")
     stream, _ = synth.generate(10, "2160p", seed=907)
-    want, got = _run_both(stream, ["-f", "yuv420", "-n", "3", "-e", "distributed"], ref_may_crash=True)
-    want = {k: v for k, v in want.items() if not k.startswith("core")}
+    args = ["-f", "yuv420", "-n", "3", "-e", "distributed"]
+    files, r = _run(MV, stream, args + ["-o", "."])
+    assert r.returncode == 0, (r.stdout[-1500:], r.stderr[-1500:])
+    got = {k: digest(v) for k, v in files.items()}
+    want = _reference_files(stream, args, may_crash=True, keep=lambda data: len(data) == 3840 * 2160 * 3 // 2)
     assert set(want) <= set(got) and len(want) >= 2
-    full = {k: v for k, v in want.items() if len(v) == 3840 * 2160 * 3 // 2}      # a file cut short by the abort does not count
+    full = {k: v for k, v in want.items() if v is not None}      # a file cut short by the abort does not count
     assert len(full) >= 2
     for name in full:
         assert full[name] == got[name], name
@@ -214,8 +224,6 @@ def test_cli_follows_parameter_set_changes_like_the_reference_cli(cli, geometry_
     with `new_size` other picture dimensions): the reference re-decodes every parameter set where it meets it
     (h264.c:128-150); mvt_extract() switches tables -- and output size -- per parameter generation."""
     from helpers import paramset_change_stream
-    if not ref.MINI_THUMBNAILER.exists():
-        pytest.skip("reference CLI not built")
     stream, segs = paramset_change_stream(geometry_change)
     want, _ = _run_both(stream, ["-f", fmt, "-n", "6"])
     assert len(want) == 6
@@ -231,21 +239,14 @@ def test_cli_skips_a_picture_it_cannot_decode_like_the_reference_cli(cli):
     both decoders refuse."""
     from helpers import PAD, split_nals
     from minivideo_b200 import synth
-    if not ref.MINI_THUMBNAILER.exists():
-        pytest.skip("reference CLI not built")
     stream, _ = synth.generate(5, width_mbs=6, height_mbs=4, profile_idc=100, transform8x8=1, seed=31)
     nals = split_nals(stream)
     bad = nals[3][:5] + bytes([0b10100000 | (nals[3][5] & 0x0f)]) + nals[3][6:]     # first_mb 0 ('1'), slice_type ue '010..'
     broken = b"".join(nals[:3] + [bad] + nals[4:]) + PAD
     good, _ = _run_both(stream, ["-f", "yuv420", "-n", "5"])
-    out = []
-    for exe, extra in ((ref.MINI_THUMBNAILER, []), (MV, ["-o", "."])):
-        with tempfile.TemporaryDirectory(dir="/dev/shm" if os.path.isdir("/dev/shm") else None) as d:
-            (Path(d) / "in.264").write_bytes(broken)
-            r = subprocess.run([str(exe), "-i", str(Path(d) / "in.264"), "-f", "yuv420", "-n", "5"] + extra,
-                               capture_output=True, text=True, cwd=d)
-            out.append(({p.name: p.read_bytes() for p in Path(d).iterdir() if p.name != "in.264"}, r))
-    (want, _), (got, r) = out
+    want = _reference_files(broken, ["-f", "yuv420", "-n", "5"], may_crash=True)
+    files, r = _run(MV, broken, ["-f", "yuv420", "-n", "5", "-o", "."])
+    got = {k: digest(v) for k, v in files.items()}
     assert sorted(want) == sorted(got) == ["in_0.yuv", "in_1.yuv", "in_2.yuv", "in_3.yuv"]
     assert want == got
     assert got["in_0.yuv"] == good["in_0.yuv"] and got["in_1.yuv"] == good["in_2.yuv"] and got["in_3.yuv"] == good["in_4.yuv"]
