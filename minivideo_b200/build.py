@@ -108,7 +108,7 @@ def build_thumbnailer(force: bool = False) -> Path:
 
 def build_oracle(force: bool = False) -> Path:
     out = ROOT / "oracle" / "librecon_oracle.so"
-    src = [ROOT / "oracle" / "recon_oracle.c", ROOT / "oracle" / "recon_oracle.h"]
+    src = [ROOT / "oracle" / "recon_oracle.c", ROOT / "oracle" / "recon_oracle.h", ROOT / "oracle" / "Makefile"]
     if force or _stale(out, src):
         _run(["make", "-C", str(ROOT / "oracle"), "oracle"] + (["-B"] if force else []))
     return out

@@ -21,8 +21,8 @@ def lib():
     global _LIB
     if _LIB is None:
         so = HERE / "librecon_oracle.so"
-        src = HERE / "recon_oracle.c"
-        if not so.exists() or so.stat().st_mtime < src.stat().st_mtime:
+        srcs = (HERE / "recon_oracle.c", HERE / "recon_oracle.h", HERE / "Makefile")
+        if not so.exists() or any(so.stat().st_mtime < s.stat().st_mtime for s in srcs):
             subprocess.run(["make", "-C", str(HERE), "oracle"], check=True, capture_output=True)
         _LIB = C.CDLL(str(so))
         _LIB.oracle_chroma_qp.restype = C.c_int

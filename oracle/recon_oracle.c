@@ -7,7 +7,8 @@
  * Differences from the reference, all outside the streams the generator emits:
  *  - Intra16x16 luma DC scaling uses the spec condition qP >= 36; the reference
  *    tests qP > 36 and executes `1 << -1` at QP'Y == 36 (h264_transform.c:797-808).
- *  - integer products/shifts wrap modulo 2^32 instead of being undefined.
+ *  - integer products, shifts and sums wrap modulo 2^32 instead of being undefined
+ *    (products and shifts through wmul/wshl, sums through -fwrapv, oracle/Makefile).
  *  - a prediction mode whose neighbours are missing predicts 0 like the
  *    reference's zero-initialised block (h264_intra_prediction.c:442,:1242);
  *    neighbour values the reference would read uninitialised are taken as 0.
