@@ -1,7 +1,7 @@
 /*
  * mvfront.h -- host front end of the intra reconstruction path (libmvfront.so).
  *
- * Written from scratch in C: Annex-B elementary-stream scan, NAL unescape, SPS / PPS /
+ * Written from scratch in C: Annex-B elementary-stream scan or MP4 sample table walk, NAL unescape, SPS / PPS /
  * slice header, CAVLC macroblock parsing -> the structure-of-arrays of mvgpu.h, one IDR
  * slice per thread.  It replaces, for this path only, what the reference does on the way
  * to its per-macroblock hot-path call (citations relative to minivideo/src/):
@@ -69,6 +69,13 @@ typedef struct mvf_batch {
  * caller reconstructs each generation's pictures with that generation's mvf_info.  FAILURE / UNSUPPORTED only
  * when no IDR picture at all has usable parameter sets. */
 int mvf_open_annexb(const uint8_t *data, size_t len, mvf_stream **out);
+/* The same stream from an MP4 / QuickTime file (ISO/IEC 14496-12) held in memory: the first video track whose
+ * sample description is avc1 / avc3.  Its NAL units are indexed in place, in the order an Annex-B stream of the same
+ * content would hold them: the avcC parameter sets of a sample description before the first sample that uses it,
+ * then every sample's length-prefixed NAL units.  Everything above then applies unchanged; mvf_select_idr() sizes a
+ * picture by its stsz sample size.  A sample whose NAL lengths run past it is skipped.  UNSUPPORTED: fragmented
+ * files, video other than H.264, no video track; FAILURE: a damaged box structure or sample table. */
+int mvf_open_mp4(const uint8_t *data, size_t len, mvf_stream **out);
 int mvf_close(mvf_stream *s);
 const char *mvf_last_error(const mvf_stream *s);      /* s may be NULL after a failed open */
 int mvf_get_info(const mvf_stream *s, mvf_info *out);                       /* generation 0 */

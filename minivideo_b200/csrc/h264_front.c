@@ -7,6 +7,7 @@
 #define _GNU_SOURCE
 #include "mvfront.h"
 
+#include <limits.h>
 #include <math.h>
 #include <pthread.h>
 #include <stdarg.h>
@@ -143,7 +144,9 @@ static inline int br_overrun(const br_t *b) { return b->pos > b->nbits; }
 
 /* ------------------------------------------------------------------------ */
 
-typedef struct { size_t off, size; int type; } nal_t;     /* off: NAL header byte */
+/* off: NAL header byte.  sample: the size mvf_select_idr() gives the picture of an IDR NAL -- the distance to the
+ * next NAL header in an Annex-B stream (esparser.c:91,:130), the stsz size of the sample that holds it in an MP4 */
+typedef struct { size_t off, size, sample; int type; } nal_t;
 
 typedef struct {
     int valid, id, err_code, profile_idc, level_idc, chroma_format_idc;
@@ -424,31 +427,46 @@ static int generation_of(mvf_stream *s, const nal_t *nl, const sps_t *sps_tab, c
     return s->n_gens++;
 }
 
+static mvf_stream *stream_new(const uint8_t *data, size_t len)
+{
+    pthread_once(&lut_once, build_luts);
+    mvf_stream *s = calloc(1, sizeof *s);
+    if (!s) return NULL;
+    s->data = data; s->len = len;
+    pthread_mutex_init(&s->err_mu, NULL);
+    return s;
+}
+
+/* room for one more entry in s->nals (*cap entries allocated); 0 when out of memory */
+static int nals_reserve(mvf_stream *s, int *cap)
+{
+    if (s->n_nals < *cap) return 1;
+    if (*cap > INT_MAX / 4) return 0;
+    const int nc = *cap ? 2 * *cap : 1024;
+    nal_t *nn = realloc(s->nals, sizeof(nal_t) * (size_t)nc);
+    if (!nn) return 0;
+    s->nals = nn; *cap = nc;
+    return 1;
+}
+
+static int index_stream(mvf_stream *s);
+
 int mvf_open_annexb(const uint8_t *data, size_t len, mvf_stream **out)
 {
     if (!out) return MVG_FAILURE;
     *out = NULL;
     if (!data || len < 5) return sfail(NULL, MVG_FAILURE, "mvf_open_annexb: empty stream");
-    pthread_once(&lut_once, build_luts);
-    mvf_stream *s = calloc(1, sizeof *s);
+    mvf_stream *s = stream_new(data, len);
     if (!s) return sfail(NULL, MVG_FAILURE, "out of memory");
-    s->data = data; s->len = len;
-    pthread_mutex_init(&s->err_mu, NULL);
 
     /* start codes 00 00 01 (a 4-byte start code is the same with one more leading zero) */
-    int cap = 1024;
-    s->nals = malloc(sizeof(nal_t) * (size_t)cap);
-    if (!s->nals) { mvf_close(s); return sfail(NULL, MVG_FAILURE, "out of memory"); }
+    int cap = 0;
     /* look for the 01 (one byte in 256 of entropy-coded data) and check the two bytes before it */
     for (const uint8_t *q = data + 2, *const end = data + len - 1; q < end; q++) {
         q = memchr(q, 1, (size_t)(end - q));
         if (!q) break;
         if (q[-1] != 0 || q[-2] != 0) continue;
-        if (s->n_nals == cap) {
-            nal_t *nn = realloc(s->nals, sizeof(nal_t) * (size_t)cap * 2);
-            if (!nn) { mvf_close(s); return sfail(NULL, MVG_FAILURE, "out of memory"); }
-            s->nals = nn; cap *= 2;
-        }
+        if (!nals_reserve(s, &cap)) { mvf_close(s); return sfail(NULL, MVG_FAILURE, "out of memory"); }
         s->nals[s->n_nals].off = (size_t)(q - data) + 1;
         s->nals[s->n_nals].type = q[1] & 31;
         s->n_nals++;
@@ -457,7 +475,17 @@ int mvf_open_annexb(const uint8_t *data, size_t len, mvf_stream **out)
         size_t end = k + 1 < s->n_nals ? s->nals[k + 1].off - 3 : len;
         while (end > s->nals[k].off && data[end - 1] == 0) end--;          /* trailing_zero_8bits */
         s->nals[k].size = end - s->nals[k].off;
+        s->nals[k].sample = (k + 1 < s->n_nals ? s->nals[k + 1].off : len) - s->nals[k].off;
     }
+    const int rc = index_stream(s);
+    if (rc == MVG_SUCCESS) *out = s;
+    return rc;
+}
+
+/* The part of opening that does not depend on the container: s->nals[] holds the NAL units in stream order.
+ * Replays the parameter sets, indexes the IDR pictures and their generations.  Closes s on failure. */
+static int index_stream(mvf_stream *s)
+{
     s->idr = malloc(sizeof(int) * (size_t)(s->n_nals + 1));
     s->idr_gen = malloc(sizeof(int) * (size_t)(s->n_nals + 1));
     sps_t *sps_tab = calloc(MVF_MAX_SPS, sizeof *sps_tab);
@@ -489,7 +517,7 @@ int mvf_open_annexb(const uint8_t *data, size_t len, mvf_stream **out)
             if (!nt) { free(tmp); free(sps_tab); free(pps_tab); mvf_close(s); return sfail(NULL, MVG_FAILURE, "out of memory"); }
             tmp = nt;
         }
-        size_t n = unescape(data + nl->off + 1, nl->size ? nl->size - 1 : 0, tmp);
+        size_t n = unescape(s->data + nl->off + 1, nl->size ? nl->size - 1 : 0, tmp);
         int id = -1, rc;
         if (nl->type == 7) {
             sps_t v;
@@ -512,8 +540,242 @@ int mvf_open_annexb(const uint8_t *data, size_t len, mvf_stream **out)
         return rc_first;
     }
     s->err[0] = 0;
-    *out = s;
     return MVG_SUCCESS;
+}
+
+/* ------------------------------------------------------------------------ */
+/* MP4 / QuickTime (ISO/IEC 14496-12, the AVC file format of 14496-15): the NAL units of the first H.264 video
+ * track, in decode order, indexed in place                                   */
+
+static uint32_t rd32(const uint8_t *p) { return (uint32_t)p[0] << 24 | (uint32_t)p[1] << 16 | (uint32_t)p[2] << 8 | p[3]; }
+static uint64_t rd64(const uint8_t *p) { return (uint64_t)rd32(p) << 32 | rd32(p + 4); }
+#define FOURCC(a, b, c, d) ((uint32_t)(a) << 24 | (uint32_t)(b) << 16 | (uint32_t)(c) << 8 | (uint32_t)(d))
+
+typedef struct { size_t body, end; } box_t;         /* payload [body, end) in the file */
+
+/* the box whose header starts at d[pos], inside a parent that ends at `end`.  0 when its header is cut short or
+ * its size is below the header or runs past the parent.  size 0 means "to the end of the parent" (of the file at
+ * the top level), size 1 a 64-bit largesize. */
+static int box_read(const uint8_t *d, size_t pos, size_t end, uint32_t *type, box_t *b)
+{
+    if (end - pos < 8) return 0;
+    uint64_t size = rd32(d + pos);
+    size_t hdr = 8;
+    *type = rd32(d + pos + 4);
+    if (size == 1) {
+        if (end - pos < 16) return 0;
+        size = rd64(d + pos + 8);
+        hdr = 16;
+    } else if (size == 0) size = end - pos;
+    if (size < hdr || size > end - pos) return 0;
+    b->body = pos + hdr; b->end = pos + (size_t)size;
+    return 1;
+}
+
+/* first child of type `want`: 1 found, 0 absent, -1 a malformed child before it */
+static int box_find(const uint8_t *d, box_t parent, uint32_t want, box_t *out)
+{
+    for (size_t pos = parent.body; pos < parent.end; pos = out->end) {
+        uint32_t t;
+        if (!box_read(d, pos, parent.end, &t, out)) return -1;
+        if (t == want) return 1;
+    }
+    return 0;
+}
+
+/* the four-character code as text, for messages */
+static const char *fourcc_str(uint32_t t, char buf[5])
+{
+    for (int i = 0; i < 4; i++) { const char c = (char)(t >> (24 - 8 * i)); buf[i] = c >= 32 && c < 127 ? c : '?'; }
+    buf[4] = 0;
+    return buf;
+}
+
+static int nal_append(mvf_stream *s, int *cap, size_t off, size_t size, size_t sample)
+{
+    if (!nals_reserve(s, cap)) return 0;
+    nal_t *nl = &s->nals[s->n_nals++];
+    nl->off = off; nl->size = size; nl->sample = sample; nl->type = s->data[off] & 31;
+    return 1;
+}
+
+/* AVCDecoderConfigurationRecord (14496-15 5.3.3.1): checks it and reads lengthSizeMinusOne; with `cap` it also
+ * appends its SPS and PPS NAL units to s->nals.  Whatever follows the PPS list (the High-profile fields) is not
+ * read.  1 = ok, 0 = malformed (message in g_open_error), -1 = out of memory. */
+static int avcc_walk(mvf_stream *s, box_t c, int *len_size, int *cap)
+{
+    const uint8_t *d = s->data;
+    if (c.end - c.body < 7) { sfail(NULL, MVG_FAILURE, "mp4: avcC box too short"); return 0; }
+    const int lsm1 = d[c.body + 4] & 3;
+    if (lsm1 == 2) { sfail(NULL, MVG_FAILURE, "mp4: avcC lengthSizeMinusOne 2 is invalid (1, 2 or 4 byte lengths)"); return 0; }
+    *len_size = lsm1 + 1;
+    size_t p = c.body + 5;
+    for (int list = 0; list < 2; list++) {
+        if (p >= c.end) { sfail(NULL, MVG_FAILURE, "mp4: avcC box truncated"); return 0; }
+        const int n = list == 0 ? d[p] & 31 : d[p];
+        p++;
+        for (int i = 0; i < n; i++) {
+            if (c.end - p < 2) { sfail(NULL, MVG_FAILURE, "mp4: avcC box truncated"); return 0; }
+            const size_t sz = (size_t)d[p] << 8 | d[p + 1];
+            p += 2;
+            if (sz > c.end - p) { sfail(NULL, MVG_FAILURE, "mp4: avcC parameter set runs past its box"); return 0; }
+            if (sz && cap && !nal_append(s, cap, p, sz, 0)) return -1;
+            p += sz;
+        }
+    }
+    return 1;
+}
+
+typedef struct { box_t avcc; int len_size; } sdesc_t;
+
+int mvf_open_mp4(const uint8_t *data, size_t len, mvf_stream **out)
+{
+    if (!out) return MVG_FAILURE;
+    *out = NULL;
+    if (!data || len < 8) return sfail(NULL, MVG_FAILURE, "mvf_open_mp4: empty file");
+    mvf_stream *s = stream_new(data, len);
+    if (!s) return sfail(NULL, MVG_FAILURE, "out of memory");
+    sdesc_t *desc = NULL;
+    int rc = MVG_FAILURE, cap = 0;
+    char cc[5];
+#define MP4_FAIL(code, ...) do { rc = sfail(NULL, code, __VA_ARGS__); goto fail; } while (0)
+
+    /* top level: ftyp, moov, mdat, ... in any order; the sample table addresses mdat by absolute file offsets */
+    box_t moov = {0, 0}, b;
+    int have_moov = 0;
+    for (size_t pos = 0; pos < len; pos = b.end) {
+        uint32_t t;
+        if (!box_read(data, pos, len, &t, &b)) MP4_FAIL(MVG_FAILURE, "mp4: truncated or overlapping box at offset %zu", pos);
+        if (t == FOURCC('m', 'o', 'o', 'f')) MP4_FAIL(MVG_UNSUPPORTED, "mp4: fragmented file (moof); only files with a complete moov index are supported");
+        if (t == FOURCC('m', 'o', 'o', 'v') && !have_moov) { moov = b; have_moov = 1; }
+    }
+    if (!have_moov) MP4_FAIL(MVG_FAILURE, "mp4: no moov box");
+
+    /* the first track whose handler is 'vide' and whose first sample description is avc1 / avc3 */
+    box_t stbl = {0, 0}, stsd = {0, 0};
+    int found = 0;
+    uint32_t other_codec = 0;
+    for (size_t pos = moov.body; pos < moov.end; pos = b.end) {
+        uint32_t t;
+        if (!box_read(data, pos, moov.end, &t, &b)) MP4_FAIL(MVG_FAILURE, "mp4: truncated or overlapping box at offset %zu", pos);
+        if (t == FOURCC('m', 'v', 'e', 'x')) MP4_FAIL(MVG_UNSUPPORTED, "mp4: fragmented file (mvex); only files with a complete moov index are supported");
+        if (t != FOURCC('t', 'r', 'a', 'k') || found) continue;
+        box_t mdia, hdlr, minf, st, sd, e;
+        int r = box_find(data, b, FOURCC('m', 'd', 'i', 'a'), &mdia);
+        if (r == 1) r = box_find(data, mdia, FOURCC('h', 'd', 'l', 'r'), &hdlr);
+        if (r < 0) MP4_FAIL(MVG_FAILURE, "mp4: truncated or overlapping box in a track");
+        if (r == 0 || hdlr.end - hdlr.body < 12 || rd32(data + hdlr.body + 8) != FOURCC('v', 'i', 'd', 'e')) continue;
+        r = box_find(data, mdia, FOURCC('m', 'i', 'n', 'f'), &minf);
+        if (r == 1) r = box_find(data, minf, FOURCC('s', 't', 'b', 'l'), &st);
+        if (r == 1) r = box_find(data, st, FOURCC('s', 't', 's', 'd'), &sd);
+        if (r < 0) MP4_FAIL(MVG_FAILURE, "mp4: truncated or overlapping box in the video track");
+        if (r == 0) MP4_FAIL(MVG_FAILURE, "mp4: video track without a sample description (stsd)");
+        uint32_t et;
+        if (sd.end - sd.body < 8 || rd32(data + sd.body + 4) == 0 || !box_read(data, sd.body + 8, sd.end, &et, &e))
+            MP4_FAIL(MVG_FAILURE, "mp4: empty or truncated sample description (stsd)");
+        if (et == FOURCC('a', 'v', 'c', '1') || et == FOURCC('a', 'v', 'c', '3')) { stbl = st; stsd = sd; found = 1; }
+        else if (!other_codec) other_codec = et;
+    }
+    if (!found && other_codec) MP4_FAIL(MVG_UNSUPPORTED, "mp4: the video track holds '%s', not H.264 (avc1 / avc3)", fourcc_str(other_codec, cc));
+    if (!found) MP4_FAIL(MVG_UNSUPPORTED, "mp4: no video track");
+
+    /* sample descriptions: every one must be H.264 with a usable avcC */
+    const uint32_t n_desc = rd32(data + stsd.body + 4);
+    if (n_desc > (stsd.end - stsd.body - 8) / 8) MP4_FAIL(MVG_FAILURE, "mp4: stsd entry count %u exceeds its box", n_desc);
+    desc = calloc(n_desc, sizeof *desc);
+    if (!desc) MP4_FAIL(MVG_FAILURE, "out of memory");
+    for (size_t pos = stsd.body + 8, i = 0; i < n_desc; i++, pos = b.end) {
+        uint32_t t;
+        box_t avcc;
+        if (!box_read(data, pos, stsd.end, &t, &b)) MP4_FAIL(MVG_FAILURE, "mp4: truncated or overlapping sample description %zu", i + 1);
+        if (t != FOURCC('a', 'v', 'c', '1') && t != FOURCC('a', 'v', 'c', '3'))
+            MP4_FAIL(MVG_UNSUPPORTED, "mp4: sample description %zu is '%s', not H.264 (avc1 / avc3)", i + 1, fourcc_str(t, cc));
+        /* VisualSampleEntry: 8 bytes of SampleEntry + 70 of visual fields, then its boxes */
+        const box_t inner = { b.body + 78, b.end };
+        if (b.end - b.body < 78 || box_find(data, inner, FOURCC('a', 'v', 'c', 'C'), &avcc) != 1)
+            MP4_FAIL(MVG_FAILURE, "mp4: sample description %zu has no readable avcC box", i + 1);
+        desc[i].avcc = avcc;
+        if (avcc_walk(s, avcc, &desc[i].len_size, NULL) != 1) goto fail;
+    }
+
+    /* sample table: sizes (stsz), samples per chunk and their description (stsc), chunk offsets (stco / co64).  Sync
+     * marks (stss) are not needed: as in an Annex-B stream, the pictures are the IDR NAL units, wherever they are. */
+    box_t stsz, stsc, stco;
+    int r = box_find(data, stbl, FOURCC('s', 't', 's', 'z'), &stsz), co64 = 0;
+    if (r == 1) r = box_find(data, stbl, FOURCC('s', 't', 's', 'c'), &stsc);
+    if (r == 1) {
+        r = box_find(data, stbl, FOURCC('s', 't', 'c', 'o'), &stco);
+        if (r == 0) { r = box_find(data, stbl, FOURCC('c', 'o', '6', '4'), &stco); co64 = 1; }
+    }
+    if (r < 0) MP4_FAIL(MVG_FAILURE, "mp4: truncated or overlapping box in the sample table");
+    if (r == 0) MP4_FAIL(MVG_FAILURE, "mp4: the sample table lacks stsz, stsc or stco / co64");
+    if (stsz.end - stsz.body < 12 || stsc.end - stsc.body < 8 || stco.end - stco.body < 8)
+        MP4_FAIL(MVG_FAILURE, "mp4: truncated stsz, stsc or chunk offset box");
+    const uint32_t const_size = rd32(data + stsz.body + 4), n_samples = rd32(data + stsz.body + 8);
+    const uint32_t n_runs = rd32(data + stsc.body + 4), n_chunks = rd32(data + stco.body + 4);
+    const size_t co_size = co64 ? 8 : 4;
+    if (const_size == 0 && n_samples > (stsz.end - stsz.body - 12) / 4) MP4_FAIL(MVG_FAILURE, "mp4: stsz sample count %u exceeds its box", n_samples);
+    if (n_samples > len) MP4_FAIL(MVG_FAILURE, "mp4: stsz sample count %u exceeds the file size", n_samples);
+    if (n_runs > (stsc.end - stsc.body - 8) / 12) MP4_FAIL(MVG_FAILURE, "mp4: stsc entry count %u exceeds its box", n_runs);
+    if (n_chunks > (stco.end - stco.body - 8) / co_size) MP4_FAIL(MVG_FAILURE, "mp4: chunk offset count %u exceeds its box", n_chunks);
+    const uint8_t *run = data + stsc.body + 8;
+    uint64_t total = 0;
+    for (uint32_t i = 0; i < n_runs; i++) {
+        const uint32_t first = rd32(run + 12 * i), per = rd32(run + 12 * i + 4), di = rd32(run + 12 * i + 8);
+        const uint64_t next = i + 1 < n_runs ? rd32(run + 12 * (i + 1)) : (uint64_t)n_chunks + 1;
+        if ((i == 0 && first != 1) || first > n_chunks || next <= first)
+            MP4_FAIL(MVG_FAILURE, "mp4: stsc entry %u: first_chunk %u (chunks must start at 1 and increase, %u chunks)", i + 1, first, n_chunks);
+        if (di < 1 || di > n_desc) MP4_FAIL(MVG_FAILURE, "mp4: stsc entry %u names sample description %u of %u", i + 1, di, n_desc);
+        total += (next - first) * per;
+        if (total > n_samples) break;
+    }
+    if (total != n_samples) MP4_FAIL(MVG_FAILURE, "mp4: stsc describes %s samples, stsz %u", total > n_samples ? "more" : "fewer", n_samples);
+
+    /* every sample in decode order: the parameter sets of its description first whenever the description changes,
+     * then its length-prefixed NAL units */
+    uint32_t sample = 0;
+    int cur_desc = -1;
+    for (uint32_t i = 0; i < n_runs; i++) {
+        const uint32_t first = rd32(run + 12 * i), per = rd32(run + 12 * i + 4), di = rd32(run + 12 * i + 8) - 1;
+        const uint64_t next = i + 1 < n_runs ? rd32(run + 12 * (i + 1)) : (uint64_t)n_chunks + 1;
+        for (uint64_t c = first; c < next && per; c++) {
+            const uint8_t *co = data + stco.body + 8 + co_size * (c - 1);
+            const uint64_t chunk = co64 ? rd64(co) : rd32(co);
+            if (chunk > len) MP4_FAIL(MVG_FAILURE, "mp4: chunk %u lies outside the file", (uint32_t)c);
+            size_t off = (size_t)chunk;
+            for (uint32_t k = 0; k < per; k++, sample++) {
+                const size_t size = const_size ? const_size : rd32(data + stsz.body + 12 + 4 * (size_t)sample);
+                if (size > len - off) MP4_FAIL(MVG_FAILURE, "mp4: sample %u lies outside the file", sample + 1);
+                if ((int)di != cur_desc) {
+                    int dummy;
+                    const int w = avcc_walk(s, desc[di].avcc, &dummy, &cap);
+                    if (w < 0) MP4_FAIL(MVG_FAILURE, "out of memory");
+                    cur_desc = (int)di;
+                }
+                /* a length field that runs past the sample drops the whole sample, like a damaged picture */
+                const int before = s->n_nals, L = desc[di].len_size;
+                for (size_t p = off, e = off + size; p < e; ) {
+                    if (e - p < (size_t)L) { s->n_nals = before; break; }
+                    size_t n = 0;
+                    for (int j = 0; j < L; j++) n = n << 8 | data[p + j];
+                    p += (size_t)L;
+                    if (n > e - p) { s->n_nals = before; break; }
+                    if (n && !nal_append(s, &cap, p, n, size)) MP4_FAIL(MVG_FAILURE, "out of memory");
+                    p += n;
+                }
+                off += size;
+            }
+        }
+    }
+    free(desc);
+#undef MP4_FAIL
+    rc = index_stream(s);
+    if (rc == MVG_SUCCESS) *out = s;
+    return rc;
+fail:
+    free(desc);
+    mvf_close(s);
+    return rc;
 }
 
 int mvf_close(mvf_stream *s)
@@ -598,15 +860,12 @@ int mvf_select_idr(const mvf_stream *s, int n_wanted, int mode, int32_t *indices
         return n_wanted;
     }
     if (n_idr < 1) return 0;
-    /* sample size = distance between NAL header bytes (esparser.c:91,:130) */
     long long payload = 0;
     long long *size = malloc(sizeof(long long) * (size_t)n_idr);
     int *cand = malloc(sizeof(int) * (size_t)n_idr), n_cand = 0;
     if (!size || !cand) { free(size); free(cand); return 0; }
     for (int i = 0; i < n_idr; i++) {
-        int k = s->idr[i];
-        size_t next = k + 1 < s->n_nals ? s->nals[k + 1].off : s->len;
-        size[i] = (long long)(next - s->nals[k].off);
+        size[i] = (long long)s->nals[s->idr[i]].sample;
         payload += size[i];
     }
     int threshold = (int)(((double)payload / (double)n_idr) / 1.66);          /* filter.c:109 */

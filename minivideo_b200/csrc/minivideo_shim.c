@@ -5,7 +5,8 @@
  *
  *   minivideo_print_infos / minivideo_get_infos / minivideo_endianness      informational
  *   minivideo_open(path, &media)      load the file                         (import.c: import_fileOpen)
- *   minivideo_parse(media, a, v, s)   Annex-B ES scan, SPS/PPS              (demuxer/esparser/esparser.c:40)
+ *   minivideo_parse(media, a, v, s)   picks the input path from the file: Annex-B ES (demuxer/esparser/esparser.c:40)
+ *                                     or MP4 / QuickTime (the reference's MP4 demuxer)
  *   minivideo_decode(media, dir, format, quality, n, mode)
  *                                     IDR selection (demuxer/filter.c:52), CAVLC on the host threads, kernels,
  *                                     picture files as export_idr() names and lays them out (export.c:618-705)
@@ -13,14 +14,16 @@
  *
  * MediaFile_t is opaque to the caller (main.cpp only passes the pointer on), so this library defines its own.
  * Scope: what this repository accelerates -- H.264 elementary streams (.264/.h264/.avc, the reference's
- * es_fileParse path), intra pictures, CAVLC, output png (also for 'jpg', as in the reference's default build) / bmp / tga /
- * yuv420 / yuv444.  Containers (AVI/MP4/MKV), webp and minivideo_extract() answer FAILURE with a message.  Like the reference (h264.c:65) pictures are written
+ * es_fileParse path) and the H.264 video track of MP4 / QuickTime files (.mp4/.m4v/.mov/.3gp/.3g2), intra pictures,
+ * CAVLC, output png (also for 'jpg', as in the reference's default build) / bmp / tga / yuv420 / yuv444.  Other
+ * containers (AVI, MKV, ...), webp and minivideo_extract() answer FAILURE with a message.  Like the reference (h264.c:65) pictures are written
  * to the current directory unless an output directory is given.  No CPU fallback.
  */
 #include <stdbool.h>
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
+#include <strings.h>
 
 #include "mv_thumbcore.h"
 
@@ -41,7 +44,7 @@ enum { PICTURE_BMP = 1, PICTURE_JPG = 2, PICTURE_PNG = 3, PICTURE_WEBP = 4, PICT
 void minivideo_print_infos(void)
 {
     printf("\nminivideo_print_infos()\n* B200 intra-reconstruction path behind the MiniVideo API (libminivideo_b200)\n"
-           "* H.264 elementary streams, CAVLC intra pictures; pictures: yuv420, bmp, tga\n\n");
+           "* H.264 elementary streams and MP4 / QuickTime files, CAVLC intra pictures; pictures: png, bmp, tga, yuv420, yuv444\n\n");
 }
 
 void minivideo_get_infos(int *major, int *minor, int *patch, const char **builddate, const char **buildtime)
@@ -91,10 +94,17 @@ int minivideo_parse(MediaFile_t *m, const bool extract_audio, const bool extract
 {
     (void)extract_audio; (void)extract_subtitles;
     if (!m || !extract_video) return FAILURE;
-    /* the reference picks its parser from the extension (import.c); only the ES path is in scope */
+    /* the reference picks its parser from the file (import.c); the ES and MP4 paths are in scope */
     const char *dot = strrchr(m->path, '.');
-    if (!dot || (strcmp(dot, ".264") && strcmp(dot, ".h264") && strcmp(dot, ".avc") && strcmp(dot, ".H264") && strcmp(dot, ".AVC"))) {
-        fprintf(stderr, "minivideo_parse: '%s' is not an H.264 elementary stream; containers are outside this library's scope\n", m->path);
+    const bool es = dot && (!strcmp(dot, ".264") || !strcmp(dot, ".h264") || !strcmp(dot, ".avc") || !strcmp(dot, ".H264") || !strcmp(dot, ".AVC"));
+    const bool mp4 = dot && (!strcasecmp(dot, ".mp4") || !strcasecmp(dot, ".m4v") || !strcasecmp(dot, ".mov") ||
+                             !strcasecmp(dot, ".3gp") || !strcasecmp(dot, ".3g2"));
+    if (mp4 && !mvt_is_mp4(m->data, m->len)) {
+        fprintf(stderr, "minivideo_parse: '%s' is not an MP4 / QuickTime file\n", m->path);
+        return FAILURE;
+    }
+    if (!es && !mp4) {
+        fprintf(stderr, "minivideo_parse: '%s' is neither an H.264 elementary stream nor an MP4 / QuickTime file; other containers are outside this library's scope\n", m->path);
         return FAILURE;
     }
     m->parsed = 1;

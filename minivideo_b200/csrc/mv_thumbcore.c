@@ -2,7 +2,7 @@
  * mv_thumbcore.c -- thumbnail extraction over the GPU path, shared by the mv_thumbnailer CLI and by the
  * drop-in public API (minivideo_shim.c):
  *
- * Annex-B bytes -> mvf_open_annexb() -> mvf_select_idr() (demuxer/filter.c semantics) ->
+ * Annex-B bytes -> mvf_open_annexb() (MP4 / QuickTime: mvf_open_mp4()) -> mvf_select_idr() (demuxer/filter.c semantics) ->
  * mvf_parse_pictures_packed() (threaded CAVLC, packed levels) -> mvg_decode_host_packed() (pinned copies +
  * kernels 0-4) -> picture
  * files named like export_idr() names them (export.c:627-642,:704-705): <input base name>[_<k>].<ext>
@@ -514,6 +514,15 @@ static int visible_gpus(void)
     return n;
 }
 
+int mvt_is_mp4(const uint8_t *data, size_t len)
+{
+    if (!data || len < 8) return 0;
+    if (!memcmp(data + 4, "ftyp", 4)) return 1;
+    const uint64_t size = (uint64_t)data[0] << 24 | (uint64_t)data[1] << 16 | (uint64_t)data[2] << 8 | data[3];
+    return size >= 8 && size <= len &&
+           (!memcmp(data + 4, "moov", 4) || !memcmp(data + 4, "mdat", 4) || !memcmp(data + 4, "free", 4) || !memcmp(data + 4, "wide", 4));
+}
+
 int mvt_extract(const uint8_t *data, size_t len, const char *base, const char *outdir, int fmt, int n_want, int mode,
                 int scale, int device, int threads, int batch, int *n_exported)
 {
@@ -522,7 +531,7 @@ int mvt_extract(const uint8_t *data, size_t len, const char *base, const char *o
     if (!outdir || !*outdir) outdir = ".";
     if (threads < 1) { long c = sysconf(_SC_NPROCESSORS_ONLN); threads = c > 0 ? (int)c : 1; }
     mvf_stream *st = NULL;
-    if (mvf_open_annexb(data, len, &st) != MVG_SUCCESS) {
+    if ((mvt_is_mp4(data, len) ? mvf_open_mp4(data, len, &st) : mvf_open_annexb(data, len, &st)) != MVG_SUCCESS) {
         fprintf(stderr, "mvt_extract: %s\n", mvf_last_error(NULL));
         return MVG_FAILURE;
     }

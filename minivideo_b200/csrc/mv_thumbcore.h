@@ -9,7 +9,11 @@
 
 enum { MVT_YUV420, MVT_BMP, MVT_TGA, MVT_PNG, MVT_YUV444 };
 
-/* Decode up to `n_want` IDR pictures of the Annex-B stream `data` (selection `mode`: 0 unfiltered, 1 ordered,
+/* Whether `data` is an MP4 / QuickTime file: bytes 4..7 are 'ftyp', or the file starts with a whole moov, mdat, free
+ * or wide box.  An Annex-B stream (00 00 00 01 ...) never is. */
+int mvt_is_mp4(const uint8_t *data, size_t len);
+
+/* Decode up to `n_want` IDR pictures of `data` -- an Annex-B stream, or an MP4 / QuickTime file (mvt_is_mp4) -- (selection `mode`: 0 unfiltered, 1 ordered,
  * 2 distributed, demuxer/filter.c:52-215) on CUDA device `device` and write them as
  * <outdir>/<base>[_<k>].{yuv,bmp,tga,png}, named and laid out like export_idr() does (export.c:627-642, :100-151,
  * :197-330, :535-601).  scale > 1 writes box-downscaled RGB thumbnails (no reference counterpart).  threads < 1: one CAVLC

@@ -2,7 +2,7 @@
  * mv_thumbnailer.c -- command-line front of the GPU path, argument-compatible with the reference's
  * mini_thumbnailer (mini_thumbnailer/src/main.cpp:77-240):
  *
- *   mv_thumbnailer -i <file.264> [-o <dir>] [-f jpg|png|bmp|tga|yuv420|yuv444] [-n N] [-e unfiltered|ordered|distributed]
+ *   mv_thumbnailer -i <file.264|file.mp4> [-o <dir>] [-f jpg|png|bmp|tga|yuv420|yuv444] [-n N] [-e unfiltered|ordered|distributed]
  *                  [-s scale] [-d device] [-t threads] [-b batch]
  *
  * The work is mvt_extract() (mv_thumbcore.c).  As in the reference's default build (no libjpeg, export.c:652-657)
@@ -20,8 +20,8 @@
 
 static void usage(void)
 {
-    fprintf(stderr, "usage: mv_thumbnailer -i <file.264> [-o <dir>] [-f jpg|png|bmp|tga|yuv420|yuv444] [-n picture_number]\n"
-                    "                      [-e unfiltered|ordered|distributed] [-s scale] [-d device] [-t threads] [-b batch]\n");
+    fprintf(stderr, "usage: mv_thumbnailer -i <file.264|file.mp4> [-o <dir>] [-f jpg|png|bmp|tga|yuv420|yuv444] [-n picture_number]\n"
+                    "                              [-e unfiltered|ordered|distributed] [-s scale] [-d device] [-t threads] [-b batch]\n");
 }
 
 int main(int argc, char **argv)

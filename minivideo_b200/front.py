@@ -1,5 +1,5 @@
-"""ctypes mirror of include/mvfront.h (libmvfront.so): the host front end that turns an Annex-B
-CAVLC intra stream into the mvgpu.h structure-of-arrays."""
+"""ctypes mirror of include/mvfront.h (libmvfront.so): the host front end that turns a CAVLC intra stream,
+Annex-B or in an MP4 / QuickTime file, into the mvgpu.h structure-of-arrays."""
 from __future__ import annotations
 
 import ctypes as C
@@ -52,6 +52,7 @@ def lib():
         _LIB = C.CDLL(str(path))
         vp = C.c_void_p
         _LIB.mvf_open_annexb.argtypes = [vp, C.c_size_t, C.POINTER(vp)]
+        _LIB.mvf_open_mp4.argtypes = [vp, C.c_size_t, C.POINTER(vp)]
         _LIB.mvf_close.argtypes = [vp]
         _LIB.mvf_last_error.argtypes = [vp]
         _LIB.mvf_last_error.restype = C.c_char_p
@@ -72,13 +73,17 @@ def lib():
 
 
 class Stream:
-    """An opened Annex-B stream (mvf_stream)."""
+    """An opened stream (mvf_stream): an Annex-B byte stream (mvf_open_annexb) or an MP4 / QuickTime file
+    (container="mp4", mvf_open_mp4)."""
 
-    def __init__(self, data: bytes):
+    def __init__(self, data: bytes, container: str = "annexb"):
         self._lib = lib()
+        opener = {"annexb": self._lib.mvf_open_annexb, "mp4": self._lib.mvf_open_mp4}.get(container)
+        if opener is None:
+            raise ValueError(f"container must be 'annexb' or 'mp4', not {container!r}")
         self._buf = np.frombuffer(data, np.uint8)          # keeps the bytes alive
         self.handle = C.c_void_p()
-        rc = self._lib.mvf_open_annexb(self._buf.ctypes.data, len(data), C.byref(self.handle))
+        rc = opener(self._buf.ctypes.data, len(data), C.byref(self.handle))
         if rc != 1:
             raise FrontError(self._lib.mvf_last_error(None).decode(), rc)
         self.info = Info()
