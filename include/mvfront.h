@@ -1,12 +1,15 @@
 /*
  * mvfront.h -- host front end of the intra reconstruction path (libmvfront.so).
  *
- * Written from scratch in C: Annex-B elementary-stream scan or MP4 sample table walk, NAL unescape, SPS / PPS /
- * slice header, CAVLC macroblock parsing -> the structure-of-arrays of mvgpu.h, one IDR
- * slice per thread.  It replaces, for this path only, what the reference does on the way
+ * Written from scratch in C: Annex-B elementary-stream scan, MP4 sample table walk, MPEG-2 transport stream demux or
+ * Matroska block walk, NAL unescape, SPS / PPS / slice header, CAVLC macroblock parsing -> the structure-of-arrays of
+ * mvgpu.h, one IDR slice per thread.  It replaces, for this path only, what the reference does on the way
  * to its per-macroblock hot-path call (citations relative to minivideo/src/):
  *
  *   es_fileParse()            demuxer/esparser/esparser.c:40     -> mvf_open_annexb()
+ *   the MP4 demuxer           demuxer/mp4/                       -> mvf_open_mp4()
+ *   the TS / PES demuxer      demuxer/mpeg/                      -> mvf_open_ts()
+ *   the Matroska demuxer      demuxer/mkv/                       -> mvf_open_mkv()
  *   idr_filtering()           demuxer/filter.c:52                -> mvf_select_idr()
  *   nalu_clean_sample()       decoder/h264/h264_nalu.c:195       -> (inside) NAL unescape
  *   decodeSPS()/decodePPS()   decoder/h264/h264_parameterset.c:123,:812
@@ -76,6 +79,27 @@ int mvf_open_annexb(const uint8_t *data, size_t len, mvf_stream **out);
  * picture by its stsz sample size.  A sample whose NAL lengths run past it is skipped.  UNSUPPORTED: fragmented
  * files, video other than H.264, no video track; FAILURE: a damaged box structure or sample table. */
 int mvf_open_mp4(const uint8_t *data, size_t len, mvf_stream **out);
+/* The same stream from an MPEG-2 transport stream (ISO/IEC 13818-1) held in memory: 188-byte packets, 192-byte M2TS
+ * packets or 204-byte packets, the size found from the sync bytes at the start (after lost sync, the next offset where
+ * the period holds again).  The first program of the PAT whose PMT lists H.264 (stream_type 0x1B) and its first such
+ * stream are taken; PSI sections must pass their CRC_32, and the first PAT / PMT that name an H.264 stream fix its PID
+ * -- later versions of either are not followed.  Concatenated, the PES payloads of that PID are an Annex-B stream, and
+ * the result is what mvf_open_annexb() gives on it: the same NAL units, pictures, generations and selection sizes.
+ * Memory: the NAL units are scattered over packets, so the stream keeps its own copy of the SPS, PPS and IDR NAL
+ * units (nothing else; mvf_close() frees it), and `data` need not outlive the call.  A continuity-counter gap, a
+ * packet with transport_error_indicator, lost sync or a cut-short PES drops the NAL units the damage touches; a
+ * duplicate packet is ignored.  UNSUPPORTED: scrambled video, video other than H.264, no video stream; FAILURE: no
+ * sync, no PAT, no PMT for the program, no PES on the video PID. */
+int mvf_open_ts(const uint8_t *data, size_t len, mvf_stream **out);
+/* The same stream from a Matroska or WebM file (EBML) held in memory: the first video TrackEntry whose CodecID is
+ * V_MPEG4/ISO/AVC.  Segment and Cluster may have unknown sizes (an unknown-size element ends at the first element that
+ * cannot be its child).  The CodecPrivate (avcC) parameter sets come before the first frame, then the frames of
+ * SimpleBlocks and BlockGroup Blocks of the track in file order, laced or not (Xiph, EBML, fixed).  Memory: as for
+ * MP4 the NAL units are indexed in place, so `data` must stay valid until mvf_close; mvf_select_idr() sizes a picture
+ * by its frame.  A frame whose NAL lengths run past it is skipped.  UNSUPPORTED: other video codecs, V_MS/VFW/FOURCC,
+ * ContentEncodings, no video track, WebM without H.264; FAILURE: a damaged EBML structure, a missing or damaged
+ * CodecPrivate, lace sizes that overrun their block. */
+int mvf_open_mkv(const uint8_t *data, size_t len, mvf_stream **out);
 int mvf_close(mvf_stream *s);
 const char *mvf_last_error(const mvf_stream *s);      /* s may be NULL after a failed open */
 int mvf_get_info(const mvf_stream *s, mvf_info *out);                       /* generation 0 */

@@ -172,6 +172,7 @@ typedef struct { sps_t sps; pps_t pps; } paramgen_t;
 
 struct mvf_stream {
     const uint8_t *data; size_t len;
+    uint8_t *own;                                           /* data when the stream holds a copy (transport streams) */
     nal_t *nals; int n_nals;
     int *idr; int n_idr;                                    /* indices into nals[] */
     int *idr_gen;                                           /* per IDR picture: its generation, or -1 (no usable SPS/PPS) */
@@ -599,29 +600,49 @@ static int nal_append(mvf_stream *s, int *cap, size_t off, size_t size, size_t s
     return 1;
 }
 
-/* AVCDecoderConfigurationRecord (14496-15 5.3.3.1): checks it and reads lengthSizeMinusOne; with `cap` it also
- * appends its SPS and PPS NAL units to s->nals.  Whatever follows the PPS list (the High-profile fields) is not
- * read.  1 = ok, 0 = malformed (message in g_open_error), -1 = out of memory. */
-static int avcc_walk(mvf_stream *s, box_t c, int *len_size, int *cap)
+/* AVCDecoderConfigurationRecord (14496-15 5.3.3.1) at [c.body, c.end) -- an MP4 avcC box or a Matroska CodecPrivate;
+ * `who` and `where` name them in messages.  Checks it and reads lengthSizeMinusOne; with `cap` it also appends its SPS
+ * and PPS NAL units to s->nals.  Whatever follows the PPS list (the High-profile fields) is not read.  1 = ok,
+ * 0 = malformed (message in g_open_error), -1 = out of memory. */
+static int avcc_walk(mvf_stream *s, const char *who, const char *where, box_t c, int *len_size, int *cap)
 {
     const uint8_t *d = s->data;
-    if (c.end - c.body < 7) { sfail(NULL, MVG_FAILURE, "mp4: avcC box too short"); return 0; }
+    if (c.end - c.body < 7) { sfail(NULL, MVG_FAILURE, "%s: avcC %s too short", who, where); return 0; }
     const int lsm1 = d[c.body + 4] & 3;
-    if (lsm1 == 2) { sfail(NULL, MVG_FAILURE, "mp4: avcC lengthSizeMinusOne 2 is invalid (1, 2 or 4 byte lengths)"); return 0; }
+    if (lsm1 == 2) { sfail(NULL, MVG_FAILURE, "%s: avcC lengthSizeMinusOne 2 is invalid (1, 2 or 4 byte lengths)", who); return 0; }
     *len_size = lsm1 + 1;
     size_t p = c.body + 5;
     for (int list = 0; list < 2; list++) {
-        if (p >= c.end) { sfail(NULL, MVG_FAILURE, "mp4: avcC box truncated"); return 0; }
+        if (p >= c.end) { sfail(NULL, MVG_FAILURE, "%s: avcC %s truncated", who, where); return 0; }
         const int n = list == 0 ? d[p] & 31 : d[p];
         p++;
         for (int i = 0; i < n; i++) {
-            if (c.end - p < 2) { sfail(NULL, MVG_FAILURE, "mp4: avcC box truncated"); return 0; }
+            if (c.end - p < 2) { sfail(NULL, MVG_FAILURE, "%s: avcC %s truncated", who, where); return 0; }
             const size_t sz = (size_t)d[p] << 8 | d[p + 1];
             p += 2;
-            if (sz > c.end - p) { sfail(NULL, MVG_FAILURE, "mp4: avcC parameter set runs past its box"); return 0; }
+            if (sz > c.end - p) { sfail(NULL, MVG_FAILURE, "%s: avcC parameter set runs past its %s", who, where); return 0; }
             if (sz && cap && !nal_append(s, cap, p, sz, 0)) return -1;
             p += sz;
         }
+    }
+    return 1;
+}
+
+/* the length-prefixed NAL units (`L`-byte lengths) of one sample / frame [off, off + size), each sized for
+ * mvf_select_idr() by the whole sample.  A length field that runs past the sample drops every NAL unit of the sample,
+ * like a damaged picture.  0 when out of memory. */
+static int sample_nals(mvf_stream *s, int *cap, size_t off, size_t size, int L)
+{
+    const uint8_t *data = s->data;
+    const int before = s->n_nals;
+    for (size_t p = off, e = off + size; p < e; ) {
+        if (e - p < (size_t)L) { s->n_nals = before; break; }
+        size_t n = 0;
+        for (int j = 0; j < L; j++) n = n << 8 | data[p + j];
+        p += (size_t)L;
+        if (n > e - p) { s->n_nals = before; break; }
+        if (n && !nal_append(s, cap, p, n, size)) return 0;
+        p += n;
     }
     return 1;
 }
@@ -695,7 +716,7 @@ int mvf_open_mp4(const uint8_t *data, size_t len, mvf_stream **out)
         if (b.end - b.body < 78 || box_find(data, inner, FOURCC('a', 'v', 'c', 'C'), &avcc) != 1)
             MP4_FAIL(MVG_FAILURE, "mp4: sample description %zu has no readable avcC box", i + 1);
         desc[i].avcc = avcc;
-        if (avcc_walk(s, avcc, &desc[i].len_size, NULL) != 1) goto fail;
+        if (avcc_walk(s, "mp4", "box", avcc, &desc[i].len_size, NULL) != 1) goto fail;
     }
 
     /* sample table: sizes (stsz), samples per chunk and their description (stsc), chunk offsets (stco / co64).  Sync
@@ -748,21 +769,11 @@ int mvf_open_mp4(const uint8_t *data, size_t len, mvf_stream **out)
                 if (size > len - off) MP4_FAIL(MVG_FAILURE, "mp4: sample %u lies outside the file", sample + 1);
                 if ((int)di != cur_desc) {
                     int dummy;
-                    const int w = avcc_walk(s, desc[di].avcc, &dummy, &cap);
+                    const int w = avcc_walk(s, "mp4", "box", desc[di].avcc, &dummy, &cap);
                     if (w < 0) MP4_FAIL(MVG_FAILURE, "out of memory");
                     cur_desc = (int)di;
                 }
-                /* a length field that runs past the sample drops the whole sample, like a damaged picture */
-                const int before = s->n_nals, L = desc[di].len_size;
-                for (size_t p = off, e = off + size; p < e; ) {
-                    if (e - p < (size_t)L) { s->n_nals = before; break; }
-                    size_t n = 0;
-                    for (int j = 0; j < L; j++) n = n << 8 | data[p + j];
-                    p += (size_t)L;
-                    if (n > e - p) { s->n_nals = before; break; }
-                    if (n && !nal_append(s, &cap, p, n, size)) MP4_FAIL(MVG_FAILURE, "out of memory");
-                    p += n;
-                }
+                if (!sample_nals(s, &cap, off, size, desc[di].len_size)) MP4_FAIL(MVG_FAILURE, "out of memory");
                 off += size;
             }
         }
@@ -778,11 +789,627 @@ fail:
     return rc;
 }
 
+/* ------------------------------------------------------------------------ */
+/* MPEG-2 transport stream (ISO/IEC 13818-1): the PES payloads of the first H.264 stream, scanned for start codes as
+ * they arrive, exactly as mvf_open_annexb() scans a stream held in one piece.  The NAL units are not contiguous in the
+ * file, so the stream keeps a copy of the ones read later -- SPS, PPS and IDR slices -- and of nothing else.      */
+
+static uint32_t crc32_mpeg(const uint8_t *p, size_t n)          /* 13818-1 Annex A: polynomial 04C11DB7, no reflection */
+{
+    uint32_t c = 0xFFFFFFFFu;
+    for (size_t i = 0; i < n; i++) {
+        c ^= (uint32_t)p[i] << 24;
+        for (int k = 0; k < 8; k++) c = c & 0x80000000u ? c << 1 ^ 0x04C11DB7u : c << 1;
+    }
+    return c;
+}
+
+/* Annex-B scan over a byte stream that arrives in pieces.  ES offsets count the bytes fed; a kept NAL unit's bytes
+ * go to buf, every other byte is only looked at. */
+typedef struct {
+    uint8_t *buf; size_t len, cap;
+    size_t pos;             /* bytes fed so far */
+    int zeros;              /* zero bytes (up to 2) at the end of what was fed since the last damage */
+    int pend;               /* the last byte fed completed 00 00 01: a start code if any byte follows */
+    int in_nal, keep, type;
+    size_t nal_es, nal_buf; /* the current NAL header byte: its ES offset and, when kept, its offset in buf */
+} es_scan;
+
+static int es_put(es_scan *e, const uint8_t *p, size_t n)
+{
+    if (!n) return 1;
+    if (e->cap - e->len < n) {
+        size_t nc = e->cap ? e->cap : 1 << 20;
+        while (nc - e->len < n) { if (nc > SIZE_MAX / 2) return 0; nc *= 2; }
+        uint8_t *nb = realloc(e->buf, nc);
+        if (!nb) return 0;
+        e->buf = nb; e->cap = nc;
+    }
+    memcpy(e->buf + e->len, p, n);
+    e->len += n;
+    return 1;
+}
+
+/* the current NAL unit ends at ES offset `end` (the start code's first zero, or the end of the stream) and the next
+ * NAL header, if any, is at `next`: the size and sample rules of mvf_open_annexb() */
+static int es_finish(mvf_stream *s, es_scan *e, int *cap, size_t end, size_t next)
+{
+    if (!e->in_nal || !e->keep) return 1;
+    size_t n = e->nal_buf + (end - e->nal_es);
+    while (n > e->nal_buf && e->buf[n - 1] == 0) n--;                  /* trailing_zero_8bits */
+    e->len = n;
+    if (!nals_reserve(s, cap)) return 0;
+    nal_t *nl = &s->nals[s->n_nals++];
+    nl->off = e->nal_buf; nl->size = n - e->nal_buf; nl->sample = next - e->nal_es; nl->type = e->type;
+    return 1;
+}
+
+static void es_start(es_scan *e, size_t off, uint8_t header)
+{
+    e->in_nal = 1;
+    e->type = header & 31;
+    e->keep = e->type == 5 || e->type == 7 || e->type == 8;
+    e->nal_es = off;
+    e->nal_buf = e->len;
+}
+
+/* lost bytes: the NAL unit they fall into is dropped, and no start code spans them; the scan resumes at the next one */
+static void es_damage(es_scan *e)
+{
+    if (e->in_nal && e->keep) e->len = e->nal_buf;
+    e->in_nal = 0; e->zeros = 0; e->pend = 0;
+}
+
+static int es_feed(mvf_stream *s, es_scan *e, int *cap, const uint8_t *c, size_t n)
+{
+    if (!n) return 1;
+    size_t from = 0;            /* c[from..) not yet copied for a kept NAL unit */
+    if (e->pend) {              /* the 01 was the last byte fed, at ES offset pos - 1 */
+        e->pend = 0;
+        if (!es_finish(s, e, cap, e->pos - 3, e->pos)) return 0;
+        es_start(e, e->pos, c[0]);
+    }
+    for (size_t i = 0; i < n; i++) {
+        const uint8_t *q = memchr(c + i, 1, n - i);
+        if (!q) break;
+        const size_t k = (size_t)(q - c);
+        i = k;
+        const int z = k >= 2 ? (c[k - 1] == 0 && c[k - 2] == 0) : k == 1 ? (c[0] == 0 && e->zeros >= 1) : e->zeros >= 2;
+        if (!z) continue;
+        if (e->in_nal && e->keep && !es_put(e, c + from, k + 1 - from)) return 0;
+        from = k + 1;
+        if (k + 1 == n) { e->pend = 1; break; }
+        if (!es_finish(s, e, cap, e->pos + k - 2, e->pos + k + 1)) return 0;
+        es_start(e, e->pos + k + 1, c[k + 1]);
+    }
+    if (e->in_nal && e->keep && !es_put(e, c + from, n - from)) return 0;
+    if (n >= 2) e->zeros = c[n - 1] ? 0 : c[n - 2] ? 1 : 2;
+    else e->zeros = c[0] ? 0 : e->zeros ? 2 : 1;
+    e->pos += n;
+    return 1;
+}
+
+/* 188-byte packets, with a 4-byte TP_extra_header before each (M2TS, 192) or 16 parity bytes after each (204): the
+ * first offset below 204 from which sync bytes repeat at one of these periods over five packets (over every whole
+ * packet of a shorter file).  0 when there is none. */
+static int ts_sync(const uint8_t *d, size_t len, size_t *first, size_t *period)
+{
+    static const size_t per[3] = {188, 192, 204};
+    for (size_t o = 0; o < 204 && o + 188 <= len; o++) {
+        if (d[o] != 0x47) continue;
+        for (int k = 0; k < 3; k++) {
+            const size_t whole = (len - o - 188) / per[k] + 1, need = whole < 5 ? whole : 5;
+            size_t i = 1;
+            while (i < need && d[o + i * per[k]] == 0x47) i++;
+            if (i == need) { *first = o; *period = per[k]; return 1; }
+        }
+    }
+    return 0;
+}
+
+/* the next packet at or after `pos`; after lost sync, the next offset at which the period holds again (for the
+ * packets that follow, as far as the file goes).  NULL at the end. */
+static const uint8_t *ts_packet(const uint8_t *d, size_t len, size_t per, size_t *pos, int *lost)
+{
+    size_t q = *pos;
+    *lost = 0;
+    if (q + 188 > len) return NULL;
+    if (d[q] != 0x47) {
+        *lost = 1;
+        for (q++; q + 188 <= len; q++)
+            if (d[q] == 0x47 && (q + per + 188 > len || d[q + per] == 0x47) && (q + 2 * per + 188 > len || d[q + 2 * per] == 0x47))
+                break;
+        if (q + 188 > len) return NULL;
+    }
+    *pos = q + per;
+    return d + q;
+}
+
+/* PSI section assembly on one PID (2.4.4): sections may span packets; 3 + section_length is at most 1024 bytes */
+typedef struct { uint8_t b[1024]; size_t have, need; int on; } psi_t;
+
+#define TS_MAX_PROGRAMS 64
+
+typedef struct {
+    int n_prog, have_pat;
+    int prog_num[TS_MAX_PROGRAMS], pmt_pid[TS_MAX_PROGRAMS];
+    int pmt_seen[TS_MAX_PROGRAMS], h264_pid[TS_MAX_PROGRAMS], other_video[TS_MAX_PROGRAMS];
+    psi_t pat, pmt[TS_MAX_PROGRAMS];
+} ts_psi;
+
+static int ts_video_type(int st)    /* stream_type values of video other than H.264 (13818-1 Table 2-34 and its amendments) */
+{
+    return st == 0x01 || st == 0x02 || st == 0x10 || st == 0x1E || st == 0x1F || st == 0x20 || st == 0x24 ||
+           st == 0x27 || st == 0x33 || st == 0x42 || st == 0xD1 || st == 0xEA;
+}
+
+/* a complete section: CRC_32 over the whole of it gives 0 (Annex A); PAT and PMT sections with current_next_indicator
+ * set are taken, the first good copy of each */
+static void ts_section(ts_psi *t, int prog, const uint8_t *b, size_t n)
+{
+    if (n < 12 || !(b[1] & 0x80) || !(b[5] & 1) || crc32_mpeg(b, n) != 0) return;
+    const size_t end = n - 4;
+    if (prog < 0) {
+        if (b[0] != 0x00 || t->have_pat) return;
+        for (size_t p = 8; p + 4 <= end && t->n_prog < TS_MAX_PROGRAMS; p += 4) {
+            const int num = b[p] << 8 | b[p + 1], pid = (b[p + 2] & 0x1F) << 8 | b[p + 3];
+            if (num == 0) continue;                         /* the network PID */
+            const int i = t->n_prog++;
+            t->prog_num[i] = num; t->pmt_pid[i] = pid;
+            t->pmt_seen[i] = 0; t->h264_pid[i] = -1; t->other_video[i] = 0;
+        }
+        t->have_pat = 1;
+        return;
+    }
+    if (b[0] != 0x02 || t->pmt_seen[prog] || (b[3] << 8 | b[4]) != t->prog_num[prog]) return;
+    size_t p = 12 + (size_t)((b[10] & 0x0F) << 8 | b[11]);           /* past program_info */
+    while (p + 5 <= end) {
+        const int st = b[p], pid = (b[p + 1] & 0x1F) << 8 | b[p + 2];
+        if (st == 0x1B && t->h264_pid[prog] < 0) t->h264_pid[prog] = pid;
+        else if (ts_video_type(st) && !t->other_video[prog]) t->other_video[prog] = st;
+        p += 5 + (size_t)((b[p + 3] & 0x0F) << 8 | b[p + 4]);
+    }
+    t->pmt_seen[prog] = 1;
+}
+
+/* one packet payload of a PSI PID */
+static void ts_psi_feed(ts_psi *t, int prog, psi_t *a, int pusi, const uint8_t *p, size_t n)
+{
+    size_t i = 0;
+    if (pusi) {
+        if (!n) return;
+        const size_t ptr = p[0];
+        i = 1;
+        if (a->on) {                                        /* the tail of the section in progress */
+            const size_t take = ptr < n - 1 ? ptr : n - 1;
+            if (a->have + take <= a->need) { memcpy(a->b + a->have, p + 1, take); a->have += take; }
+            if (a->have == a->need) ts_section(t, prog, a->b, a->need);
+        }
+        a->on = 0;
+        i += ptr;
+        while (i < n && p[i] != 0xFF) {                     /* sections that start here; 0xFF is stuffing */
+            if (n - i < 3) { memcpy(a->b, p + i, n - i); a->have = n - i; a->need = 0; a->on = 1; return; }
+            const size_t need = 3 + (size_t)((p[i + 1] & 0x0F) << 8 | p[i + 2]);
+            if (need > sizeof a->b) return;
+            if (n - i >= need) { ts_section(t, prog, p + i, need); i += need; continue; }
+            memcpy(a->b, p + i, n - i); a->have = n - i; a->need = need; a->on = 1;
+            return;
+        }
+        return;
+    }
+    if (!a->on) return;
+    if (a->need == 0) {                                     /* the section header itself was split */
+        const size_t take = 3 - a->have < n ? 3 - a->have : n;
+        memcpy(a->b + a->have, p, take); a->have += take; p += take; n -= take;
+        if (a->have < 3) return;
+        a->need = 3 + (size_t)((a->b[1] & 0x0F) << 8 | a->b[2]);
+        if (a->need > sizeof a->b) { a->on = 0; return; }
+    }
+    const size_t take = a->need - a->have < n ? a->need - a->have : n;
+    memcpy(a->b + a->have, p, take);
+    a->have += take;
+    if (a->have == a->need) { ts_section(t, prog, a->b, a->need); a->on = 0; }
+}
+
+/* the chosen program once it is certain: the first program of the PAT whose PMT lists H.264, all earlier ones seen */
+static int ts_choice(const ts_psi *t, int at_end)
+{
+    for (int i = 0; i < t->n_prog; i++) {
+        if (t->pmt_seen[i] && t->h264_pid[i] >= 0) return i;
+        if (!t->pmt_seen[i] && !at_end) return -1;
+    }
+    return -1;
+}
+
+int mvf_open_ts(const uint8_t *data, size_t len, mvf_stream **out)
+{
+    if (!out) return MVG_FAILURE;
+    *out = NULL;
+    size_t first, per;
+    if (!data || !ts_sync(data, len, &first, &per)) return sfail(NULL, MVG_FAILURE, "ts: no sync bytes at a 188, 192 or 204 byte period");
+    ts_psi *t = calloc(1, sizeof *t);
+    mvf_stream *s = stream_new(data, len);
+    es_scan e;
+    memset(&e, 0, sizeof e);
+    int rc = MVG_FAILURE, cap = 0;
+#define TS_FAIL(code, ...) do { rc = sfail(NULL, code, __VA_ARGS__); goto fail; } while (0)
+    if (!s || !t) TS_FAIL(MVG_FAILURE, "out of memory");
+
+    /* pass 1: PAT and PMTs, until the choice is certain or the file ends */
+    int lost, prog = -1;
+    const uint8_t *pk;
+    for (size_t pos = first; prog < 0 && (pk = ts_packet(data, len, per, &pos, &lost)); ) {
+        const int pid = (pk[1] & 0x1F) << 8 | pk[2], afc = pk[3] >> 4 & 3;
+        if (pk[1] & 0x80 || !(afc & 1)) continue;
+        const size_t o = afc & 2 ? 5 + (size_t)pk[4] : 4;
+        if (o >= 188) continue;
+        if (pid == 0) ts_psi_feed(t, -1, &t->pat, pk[1] & 0x40, pk + o, 188 - o);
+        else
+            for (int i = 0; i < t->n_prog; i++)
+                if (t->pmt_pid[i] == pid) ts_psi_feed(t, i, &t->pmt[i], pk[1] & 0x40, pk + o, 188 - o);
+        if (t->have_pat) prog = ts_choice(t, 0);
+    }
+    if (!t->have_pat) TS_FAIL(MVG_FAILURE, "ts: no program association table (PAT)");
+    if (prog < 0) prog = ts_choice(t, 1);
+    if (prog < 0) {
+        for (int i = 0; i < t->n_prog; i++)
+            if (t->other_video[i])
+                TS_FAIL(MVG_UNSUPPORTED, "ts: program %d carries video of stream_type 0x%02X, not H.264 (0x1B)", t->prog_num[i], t->other_video[i]);
+        for (int i = 0; i < t->n_prog; i++)
+            if (!t->pmt_seen[i]) TS_FAIL(MVG_FAILURE, "ts: no program map table (PMT) for program %d on PID 0x%X", t->prog_num[i], t->pmt_pid[i]);
+        TS_FAIL(MVG_UNSUPPORTED, "ts: no video stream in %s", t->n_prog ? "any program" : "the PAT (it lists no program)");
+    }
+    const int vpid = t->h264_pid[prog];
+
+    /* pass 2: the PES packets of that PID from the start of the file */
+    int last_cc = -1, dup = 0, in_hdr = 0, in_pes = 0, bounded = 0;
+    size_t hlen = 0, left = 0, n_pes = 0;
+    uint8_t hdr[9 + 255];
+    /* Lost bytes (lost sync, a continuity gap, an errored packet) drop the NAL unit they fall into.  What follows on
+     * the PID up to the next payload_unit_start_indicator is still payload of one PES packet, so it is scanned on, but
+     * that packet's length no longer says anything; only a PES header cut in two loses the rest of its packet. */
+#define TS_DAMAGE() do { es_damage(&e); if (in_hdr) in_hdr = in_pes = 0; else { in_pes = n_pes > 0; bounded = 0; } } while (0)
+    for (size_t pos = first; (pk = ts_packet(data, len, per, &pos, &lost)); ) {
+        if (lost) TS_DAMAGE();
+        const int pid = (pk[1] & 0x1F) << 8 | pk[2];
+        if (pk[1] & 0x80) {                                 /* transport_error_indicator: the packet cannot be trusted */
+            if (pid == vpid) TS_DAMAGE();
+            continue;
+        }
+        if (pid != vpid) continue;
+        if (pk[3] >> 6) TS_FAIL(MVG_UNSUPPORTED, "ts: the video packets are scrambled (transport_scrambling_control %d)", pk[3] >> 6);
+        const int afc = pk[3] >> 4 & 3, cc = pk[3] & 15;
+        size_t o = 4;
+        int disc = 0;
+        if (afc & 2) {
+            o = 5 + (size_t)pk[4];
+            disc = pk[4] && (pk[5] & 0x80);                 /* discontinuity_indicator */
+        }
+        if (!(afc & 1)) continue;                           /* no payload: the counter does not advance */
+        if (last_cc >= 0 && cc == last_cc && !dup && !disc) { dup = 1; continue; }     /* a duplicate packet */
+        const int gap = last_cc >= 0 && cc != ((last_cc + 1) & 15) && !disc;
+        last_cc = cc; dup = 0;
+        if (gap || o > 188) {
+            TS_DAMAGE();
+            if (o > 188) continue;
+        }
+        const uint8_t *p = pk + o;
+        size_t n = 188 - o;
+        if (pk[1] & 0x40) {                                 /* payload_unit_start_indicator: a new PES packet */
+            if ((in_pes && bounded && left) || in_hdr) es_damage(&e);          /* the previous one was cut short */
+            in_pes = 0; in_hdr = 1; hlen = 0;
+        }
+        if (in_hdr) {
+            const size_t want = hlen < 9 ? 9 : 9 + (size_t)hdr[8];
+            size_t take = want - hlen < n ? want - hlen : n;
+            memcpy(hdr + hlen, p, take); hlen += take; p += take; n -= take;
+            if (hlen == 9 && hdr[8] && n) {
+                take = hdr[8] < n ? hdr[8] : n;
+                memcpy(hdr + hlen, p, take); hlen += take; p += take; n -= take;
+            }
+            if (hlen < 9 || hlen < 9 + (size_t)hdr[8]) continue;
+            in_hdr = 0;
+            if (hdr[0] || hdr[1] || hdr[2] != 1 || hdr[3] < 0xE0 || hdr[3] > 0xEF || (hdr[6] & 0xC0) != 0x80) {
+                es_damage(&e);                              /* not a video PES header */
+                continue;
+            }
+            if (hdr[6] >> 4 & 3) TS_FAIL(MVG_UNSUPPORTED, "ts: the video PES packets are scrambled (PES_scrambling_control %d)", hdr[6] >> 4 & 3);
+            const size_t plen = (size_t)hdr[4] << 8 | hdr[5];
+            bounded = plen != 0;
+            if (bounded && plen < 3 + (size_t)hdr[8]) { es_damage(&e); continue; }
+            left = bounded ? plen - 3 - hdr[8] : 0;
+            in_pes = 1; n_pes++;
+        }
+        if (!in_pes) continue;
+        if (bounded) {
+            if (n > left) n = left;
+            left -= n;
+        }
+        if (!es_feed(s, &e, &cap, p, n)) TS_FAIL(MVG_FAILURE, "out of memory");
+        if (bounded && !left) in_pes = 0;
+    }
+    if ((in_pes && bounded && left) || in_hdr) es_damage(&e);
+#undef TS_DAMAGE
+    if (!n_pes) TS_FAIL(MVG_FAILURE, "ts: the H.264 stream of program %d (PID 0x%X) carries no PES packet", t->prog_num[prog], vpid);
+    if (!es_finish(s, &e, &cap, e.pos, e.pos)) TS_FAIL(MVG_FAILURE, "out of memory");
+#undef TS_FAIL
+    free(t);
+    {   /* the copy is final: give back the unused capacity, and point the stream at it */
+        uint8_t *b = e.len ? realloc(e.buf, e.len) : e.buf;
+        if (b) e.buf = b;
+    }
+    s->data = s->own = e.buf; s->len = e.len;
+    rc = index_stream(s);
+    if (rc == MVG_SUCCESS) *out = s;
+    return rc;
+fail:
+    free(t); free(e.buf);
+    if (s) mvf_close(s);
+    return rc;
+}
+
+/* ------------------------------------------------------------------------ */
+/* Matroska / WebM (EBML, RFC 8794; Matroska, RFC 9559): the frames of the first H.264 video track, in file order, their
+ * length-prefixed NAL units indexed in place                                  */
+
+#define MKV_SEGMENT      0x18538067u
+#define MKV_CLUSTER      0x1F43B675u
+#define MKV_TRACKS       0x1654AE6Bu
+
+/* an EBML variable-length integer at d[*pos]: an element ID keeps its length marker (1..4 bytes), a size loses it
+ * (1..8 bytes; all value bits set = unknown, returned as UINT64_MAX).  0 when it is cut short or too wide. */
+static int ebml_vint(const uint8_t *d, size_t *pos, size_t end, int is_id, uint64_t *v)
+{
+    if (*pos >= end || !d[*pos]) return 0;
+    const int w = __builtin_clz(d[*pos]) - 23;
+    if (w > (is_id ? 4 : 8) || end - *pos < (size_t)w) return 0;
+    uint64_t x = is_id ? d[*pos] : d[*pos] & (0xFFu >> w);
+    for (int i = 1; i < w; i++) x = x << 8 | d[*pos + i];
+    *pos += (size_t)w;
+    *v = !is_id && x == (1ull << (7 * w)) - 1 ? UINT64_MAX : x;
+    return 1;
+}
+
+typedef struct { uint32_t id; size_t body, end; int unknown; } ebml_t;
+
+/* the element at d[pos] inside a parent that ends at `end`; an unknown size reaches to `end` for now.  0 when its
+ * header is cut short or its size runs past the parent. */
+static int ebml_read(const uint8_t *d, size_t pos, size_t end, ebml_t *e)
+{
+    uint64_t id, size;
+    if (!ebml_vint(d, &pos, end, 1, &id) || !ebml_vint(d, &pos, end, 0, &size)) return 0;
+    e->id = (uint32_t)id; e->body = pos;
+    e->unknown = size == UINT64_MAX;
+    if (!e->unknown && size > end - pos) return 0;
+    e->end = e->unknown ? end : pos + (size_t)size;
+    return 1;
+}
+
+static uint64_t ebml_uint(const uint8_t *d, ebml_t e)
+{
+    uint64_t v = 0;
+    for (size_t p = e.body; p < e.end && p < e.body + 8; p++) v = v << 8 | d[p];
+    return v;
+}
+
+static int ebml_is(const uint8_t *d, ebml_t e, const char *str)
+{
+    const size_t n = strlen(str);
+    size_t m = e.end - e.body;
+    while (m > 0 && d[e.body + m - 1] == 0) m--;            /* strings may be zero-padded */
+    return m == n && !memcmp(d + e.body, str, n);
+}
+
+static int mkv_segment_child(uint32_t id)
+{
+    return id == 0x114D9B74u || id == 0x1549A966u || id == MKV_TRACKS || id == MKV_CLUSTER || id == 0x1C53BB6Bu ||
+           id == 0x1941A469u || id == 0x1043A770u || id == 0x1254C367u || id == 0xECu || id == 0xBFu;
+}
+
+static int mkv_cluster_child(uint32_t id)
+{
+    return id == 0xE7u || id == 0x5854u || id == 0xA7u || id == 0xABu || id == 0xA3u || id == 0xA0u || id == 0xAFu ||
+           id == 0xECu || id == 0xBFu;
+}
+
+typedef struct { uint64_t number; int len_size, replayed; box_t priv; } mkv_track;
+
+/* the frames of a SimpleBlock or Block [b, end) of the track: header, lacing (Xiph, EBML, fixed), then each frame's NAL
+ * units.  Returns 1, or a return code with a message for a damaged block or when out of memory. */
+static int mkv_block(mvf_stream *s, mkv_track *tr, size_t b, size_t end, int *cap)
+{
+    const uint8_t *d = s->data;
+    uint64_t tn;
+    size_t p = b;
+    if (!ebml_vint(d, &p, end, 0, &tn) || end - p < 3) return sfail(NULL, MVG_FAILURE, "mkv: truncated block header at offset %zu", b);
+    if (tn != tr->number) return 1;
+    const int lacing = d[p + 2] >> 1 & 3;
+    p += 3;
+    size_t sizes[256];
+    int count = 1;
+    if (lacing) {
+        if (p >= end) return sfail(NULL, MVG_FAILURE, "mkv: lace sizes overrun their block at offset %zu", b);
+        count = d[p++] + 1;
+        if (lacing == 2) {                                  /* fixed */
+            if ((end - p) % (size_t)count) return sfail(NULL, MVG_FAILURE, "mkv: lace sizes overrun their block at offset %zu", b);
+            for (int i = 0; i < count; i++) sizes[i] = (end - p) / (size_t)count;
+        } else {
+            size_t sum = 0;
+            for (int i = 0; i < count - 1; i++) {
+                uint64_t v = 0;
+                if (lacing == 1) {                          /* Xiph: 255s and a final byte */
+                    uint8_t c;
+                    do {
+                        if (p >= end) return sfail(NULL, MVG_FAILURE, "mkv: lace sizes overrun their block at offset %zu", b);
+                        c = d[p++]; v += c;
+                    } while (c == 255);
+                } else {                                    /* EBML: a size, then signed differences */
+                    const size_t at = p;
+                    if (!ebml_vint(d, &p, end, 0, &v) || v == UINT64_MAX)
+                        return sfail(NULL, MVG_FAILURE, "mkv: lace sizes overrun their block at offset %zu", b);
+                    if (i > 0) {
+                        const int w = (int)(p - at);
+                        const int64_t delta = (int64_t)v - (int64_t)((1ull << (7 * w - 1)) - 1);
+                        if ((int64_t)sizes[i - 1] + delta < 0) return sfail(NULL, MVG_FAILURE, "mkv: lace sizes overrun their block at offset %zu", b);
+                        v = (uint64_t)((int64_t)sizes[i - 1] + delta);
+                    }
+                }
+                if (v > end - p || sum + v > end - p) return sfail(NULL, MVG_FAILURE, "mkv: lace sizes overrun their block at offset %zu", b);
+                sizes[i] = (size_t)v; sum += (size_t)v;
+            }
+            if (sum > end - p) return sfail(NULL, MVG_FAILURE, "mkv: lace sizes overrun their block at offset %zu", b);
+            sizes[count - 1] = end - p - sum;
+        }
+    } else sizes[0] = end - p;
+    for (int i = 0; i < count; i++) {
+        if (!tr->replayed) {                                /* the CodecPrivate parameter sets before the first frame */
+            int dummy;
+            if (avcc_walk(s, "mkv", "CodecPrivate", tr->priv, &dummy, cap) < 0) return sfail(NULL, MVG_FAILURE, "out of memory");
+            tr->replayed = 1;
+        }
+        if (!sample_nals(s, cap, p, sizes[i], tr->len_size)) return sfail(NULL, MVG_FAILURE, "out of memory");
+        p += sizes[i];
+    }
+    return 1;
+}
+
+/* the next child of a Segment from `pos` (which ends at `end`): 1 with *e, 0 at its end, -1 damaged.  An unknown-size
+ * Segment ends at the first element that cannot be its child; an unknown-size Cluster at the first one that cannot be
+ * the Cluster's, and its end is found by walking it. */
+static int mkv_next(const uint8_t *d, size_t pos, size_t end, int seg_unknown, ebml_t *e)
+{
+    if (pos >= end) return 0;
+    if (!ebml_read(d, pos, end, e)) return -1;
+    if (seg_unknown && !mkv_segment_child(e->id)) return 0;
+    if (e->unknown) {
+        if (e->id != MKV_CLUSTER) return -1;
+        ebml_t c;
+        size_t p = e->body;
+        while (p < end) {
+            if (!ebml_read(d, p, end, &c)) return -1;
+            if (!mkv_cluster_child(c.id)) break;
+            if (c.unknown) return -1;
+            p = c.end;
+        }
+        e->end = p;
+    }
+    return 1;
+}
+
+int mvf_open_mkv(const uint8_t *data, size_t len, mvf_stream **out)
+{
+    if (!out) return MVG_FAILURE;
+    *out = NULL;
+    if (!data || len < 4 || rd32(data) != 0x1A45DFA3u) return sfail(NULL, MVG_FAILURE, "mkv: no EBML header");
+    mvf_stream *s = stream_new(data, len);
+    if (!s) return sfail(NULL, MVG_FAILURE, "out of memory");
+    int rc = MVG_FAILURE, cap = 0;
+#define MKV_FAIL(code, ...) do { rc = sfail(NULL, code, __VA_ARGS__); goto fail; } while (0)
+
+    /* EBML header (its DocType), then the first Segment */
+    ebml_t e, seg = {0, 0, 0, 0};
+    int webm = 0, have_seg = 0;
+    if (!ebml_read(data, 0, len, &e) || e.unknown) MKV_FAIL(MVG_FAILURE, "mkv: damaged EBML header");
+    for (size_t p = e.body; p < e.end; ) {
+        ebml_t c;
+        if (!ebml_read(data, p, e.end, &c) || c.unknown) MKV_FAIL(MVG_FAILURE, "mkv: damaged EBML header");
+        if (c.id == 0x4282u) webm = ebml_is(data, c, "webm");               /* DocType */
+        p = c.end;
+    }
+    for (size_t p = e.end; p < len && !have_seg; ) {
+        if (!ebml_read(data, p, len, &seg)) MKV_FAIL(MVG_FAILURE, "mkv: damaged element at offset %zu", p);
+        if (seg.id == MKV_SEGMENT) have_seg = 1;
+        else if (seg.unknown) MKV_FAIL(MVG_FAILURE, "mkv: element of unknown size at offset %zu", p);
+        else p = seg.end;
+    }
+    if (!have_seg) MKV_FAIL(MVG_FAILURE, "mkv: no Segment");
+
+    /* the first Tracks element: the first TrackEntry of type video (1) whose CodecID is V_MPEG4/ISO/AVC */
+    mkv_track tr;
+    memset(&tr, 0, sizeof tr);
+    int found = 0, r;
+    char other[64] = "";
+    for (size_t p = seg.body; (r = mkv_next(data, p, seg.end, seg.unknown, &e)) == 1 && !found; p = e.end) {
+        if (e.id != MKV_TRACKS) continue;
+        for (size_t q = e.body; q < e.end && !found; ) {
+            ebml_t te;
+            if (!ebml_read(data, q, e.end, &te) || te.unknown) MKV_FAIL(MVG_FAILURE, "mkv: damaged Tracks element at offset %zu", q);
+            q = te.end;
+            if (te.id != 0xAEu) continue;                   /* TrackEntry */
+            uint64_t number = 0, type = 0;
+            int avc = 0, encoded = 0, have_priv = 0;
+            ebml_t codec = {0, 0, 0, 0}, priv = {0, 0, 0, 0};
+            for (size_t k = te.body; k < te.end; ) {
+                ebml_t c;
+                if (!ebml_read(data, k, te.end, &c) || c.unknown) MKV_FAIL(MVG_FAILURE, "mkv: damaged TrackEntry at offset %zu", k);
+                if (c.id == 0xD7u) number = ebml_uint(data, c);
+                else if (c.id == 0x83u) type = ebml_uint(data, c);
+                else if (c.id == 0x86u) { codec = c; avc = ebml_is(data, c, "V_MPEG4/ISO/AVC"); }
+                else if (c.id == 0x63A2u) { priv = c; have_priv = 1; }
+                else if (c.id == 0x6D80u) encoded = 1;      /* ContentEncodings */
+                k = c.end;
+            }
+            if (type != 1) continue;
+            if (!avc) {
+                if (!other[0]) {
+                    size_t n = codec.end - codec.body < sizeof other - 1 ? codec.end - codec.body : sizeof other - 1;
+                    for (size_t i = 0; i < n; i++) { const char ch = (char)data[codec.body + i]; other[i] = ch >= 32 && ch < 127 ? ch : '?'; }
+                    other[n] = 0;
+                    if (!n) snprintf(other, sizeof other, "no CodecID");
+                }
+                continue;
+            }
+            if (encoded) MKV_FAIL(MVG_UNSUPPORTED, "mkv: the H.264 track has ContentEncodings (compressed or encrypted frames)");
+            if (!number) MKV_FAIL(MVG_FAILURE, "mkv: the H.264 track has no TrackNumber");
+            if (!have_priv) MKV_FAIL(MVG_FAILURE, "mkv: the H.264 track has no CodecPrivate (avcC)");
+            tr.number = number;
+            tr.priv = (box_t){priv.body, priv.end};
+            const int w = avcc_walk(s, "mkv", "CodecPrivate", tr.priv, &tr.len_size, NULL);
+            if (w != 1) { rc = MVG_FAILURE; goto fail; }
+            found = 1;
+        }
+    }
+    if (r < 0) MKV_FAIL(MVG_FAILURE, "mkv: damaged EBML structure in the Segment");
+    if (!found && !strcmp(other, "V_MS/VFW/FOURCC"))
+        MKV_FAIL(MVG_UNSUPPORTED, "mkv: the video track is V_MS/VFW/FOURCC (Video for Windows); only V_MPEG4/ISO/AVC is supported");
+    if (!found && other[0]) MKV_FAIL(MVG_UNSUPPORTED, "mkv: the video track holds %s, not H.264 (V_MPEG4/ISO/AVC)", other);
+    if (!found && webm) MKV_FAIL(MVG_UNSUPPORTED, "mkv: WebM file without an H.264 video track");
+    if (!found) MKV_FAIL(MVG_UNSUPPORTED, "mkv: no video track");
+
+    /* every Cluster in file order: SimpleBlocks, and Blocks inside BlockGroups, of that track */
+    for (size_t p = seg.body; (r = mkv_next(data, p, seg.end, seg.unknown, &e)) == 1; p = e.end) {
+        if (e.id != MKV_CLUSTER) continue;
+        for (size_t q = e.body; q < e.end; ) {
+            ebml_t c;
+            if (!ebml_read(data, q, e.end, &c) || c.unknown) MKV_FAIL(MVG_FAILURE, "mkv: damaged Cluster at offset %zu", q);
+            q = c.end;
+            int br = 1;
+            if (c.id == 0xA3u) br = mkv_block(s, &tr, c.body, c.end, &cap);             /* SimpleBlock */
+            else if (c.id == 0xA0u)                                                     /* BlockGroup */
+                for (size_t k = c.body; k < c.end && br == 1; ) {
+                    ebml_t bl;
+                    if (!ebml_read(data, k, c.end, &bl) || bl.unknown) MKV_FAIL(MVG_FAILURE, "mkv: damaged BlockGroup at offset %zu", k);
+                    if (bl.id == 0xA1u) br = mkv_block(s, &tr, bl.body, bl.end, &cap);  /* Block */
+                    k = bl.end;
+                }
+            if (br != 1) { rc = br; goto fail; }
+        }
+    }
+    if (r < 0) MKV_FAIL(MVG_FAILURE, "mkv: damaged EBML structure in the Segment");
+#undef MKV_FAIL
+    rc = index_stream(s);
+    if (rc == MVG_SUCCESS) *out = s;
+    return rc;
+fail:
+    mvf_close(s);
+    return rc;
+}
+
 int mvf_close(mvf_stream *s)
 {
     if (!s) return MVG_FAILURE;
     pthread_mutex_destroy(&s->err_mu);
-    free(s->nals); free(s->idr); free(s->idr_gen); free(s->gens); free(s);
+    free(s->nals); free(s->idr); free(s->idr_gen); free(s->gens); free(s->own); free(s);
     return MVG_SUCCESS;
 }
 

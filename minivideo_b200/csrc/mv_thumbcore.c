@@ -2,7 +2,8 @@
  * mv_thumbcore.c -- thumbnail extraction over the GPU path, shared by the mv_thumbnailer CLI and by the
  * drop-in public API (minivideo_shim.c):
  *
- * Annex-B bytes -> mvf_open_annexb() (MP4 / QuickTime: mvf_open_mp4()) -> mvf_select_idr() (demuxer/filter.c semantics) ->
+ * Annex-B bytes -> mvf_open_annexb() (MP4 / QuickTime, transport streams, Matroska: mvf_open_mp4() / _ts() / _mkv(),
+ * picked by mvt_container()) -> mvf_select_idr() (demuxer/filter.c semantics) ->
  * mvf_parse_pictures_packed() (threaded CAVLC, packed levels) -> mvg_decode_host_packed() (pinned copies +
  * kernels 0-4) -> picture
  * files named like export_idr() names them (export.c:627-642,:704-705): <input base name>[_<k>].<ext>
@@ -523,6 +524,25 @@ int mvt_is_mp4(const uint8_t *data, size_t len)
            (!memcmp(data + 4, "moov", 4) || !memcmp(data + 4, "mdat", 4) || !memcmp(data + 4, "free", 4) || !memcmp(data + 4, "wide", 4));
 }
 
+int mvt_container(const uint8_t *data, size_t len)
+{
+    if (mvt_is_mp4(data, len)) return MVT_CONTAINER_MP4;       /* first, as before there were other containers */
+    if (!data || len < 4) return MVT_ANNEXB;
+    if ((data[0] == 0 && data[1] == 0 && data[2] == 1) || (data[0] == 0 && data[1] == 0 && data[2] == 0 && data[3] == 1))
+        return MVT_ANNEXB;
+    if (data[0] == 0x1A && data[1] == 0x45 && data[2] == 0xDF && data[3] == 0xA3) return MVT_CONTAINER_MKV;
+    static const size_t per[3] = {188, 192, 204};
+    for (size_t o = 0; o < 204 && o + 4 * 204 < len; o++) {
+        if (data[o] != 0x47) continue;
+        for (int k = 0; k < 3; k++) {
+            int i = 1;
+            while (i < 5 && data[o + (size_t)i * per[k]] == 0x47) i++;
+            if (i == 5) return MVT_CONTAINER_TS;
+        }
+    }
+    return MVT_ANNEXB;
+}
+
 int mvt_extract(const uint8_t *data, size_t len, const char *base, const char *outdir, int fmt, int n_want, int mode,
                 int scale, int device, int threads, int batch, int *n_exported)
 {
@@ -531,8 +551,12 @@ int mvt_extract(const uint8_t *data, size_t len, const char *base, const char *o
     if (!outdir || !*outdir) outdir = ".";
     if (threads < 1) { long c = sysconf(_SC_NPROCESSORS_ONLN); threads = c > 0 ? (int)c : 1; }
     mvf_stream *st = NULL;
-    if ((mvt_is_mp4(data, len) ? mvf_open_mp4(data, len, &st) : mvf_open_annexb(data, len, &st)) != MVG_SUCCESS) {
-        fprintf(stderr, "mvt_extract: %s\n", mvf_last_error(NULL));
+    int (*const open[4])(const uint8_t *, size_t, mvf_stream **) = {
+        [MVT_ANNEXB] = mvf_open_annexb, [MVT_CONTAINER_MP4] = mvf_open_mp4, [MVT_CONTAINER_TS] = mvf_open_ts, [MVT_CONTAINER_MKV] = mvf_open_mkv };
+    static const char *const kind[4] = {"an H.264 elementary stream", "an MP4 / QuickTime file", "an MPEG-2 transport stream", "a Matroska / WebM file"};
+    const int container = mvt_container(data, len);
+    if (open[container](data, len, &st) != MVG_SUCCESS) {
+        fprintf(stderr, "mvt_extract: cannot read the input as %s: %s\n", kind[container], mvf_last_error(NULL));
         return MVG_FAILURE;
     }
     mvf_info info;

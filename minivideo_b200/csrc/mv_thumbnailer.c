@@ -2,9 +2,11 @@
  * mv_thumbnailer.c -- command-line front of the GPU path, argument-compatible with the reference's
  * mini_thumbnailer (mini_thumbnailer/src/main.cpp:77-240):
  *
- *   mv_thumbnailer -i <file.264|file.mp4> [-o <dir>] [-f jpg|png|bmp|tga|yuv420|yuv444] [-n N] [-e unfiltered|ordered|distributed]
+ *   mv_thumbnailer -i <file.264|.mp4|.ts|.m2ts|.mkv> [-o <dir>] [-f jpg|png|bmp|tga|yuv420|yuv444] [-n N] [-e unfiltered|ordered|distributed]
  *                  [-s scale] [-d device] [-t threads] [-b batch]
  *
+ * The input is an H.264 elementary stream, an MP4 / QuickTime file, an MPEG-2 transport stream (188, 192 or 204-byte
+ * packets) or a Matroska / WebM file, told apart by content (mvt_container), not by name.
  * The work is mvt_extract() (mv_thumbcore.c).  As in the reference's default build (no libjpeg, export.c:652-657)
  * 'jpg' -- also the default format, main.cpp:56 -- is written as PNG.  Extensions over the reference: -o is honoured (the reference
  * ignores it, h264.c:65), -s writes a box-downscaled RGB thumbnail, -d/-t/-b pick the GPU, parser threads and
@@ -20,8 +22,9 @@
 
 static void usage(void)
 {
-    fprintf(stderr, "usage: mv_thumbnailer -i <file.264|file.mp4> [-o <dir>] [-f jpg|png|bmp|tga|yuv420|yuv444] [-n picture_number]\n"
-                    "                              [-e unfiltered|ordered|distributed] [-s scale] [-d device] [-t threads] [-b batch]\n");
+    fprintf(stderr, "usage: mv_thumbnailer -i <file.264|.mp4|.mov|.ts|.m2ts|.mkv|.webm> [-o <dir>] [-f jpg|png|bmp|tga|yuv420|yuv444]\n"
+                    "                      [-n picture_number] [-e unfiltered|ordered|distributed] [-s scale] [-d device] [-t threads] [-b batch]\n"
+                    "  input: H.264 elementary stream, MP4 / QuickTime, MPEG-2 transport stream or Matroska / WebM (found from the content)\n");
 }
 
 int main(int argc, char **argv)

@@ -42,6 +42,11 @@ class FrontError(RuntimeError):
         self.code = code
 
 
+class OpenError(FrontError, ValueError):
+    """The bytes given to Stream cannot be opened as the container named: a bad argument value, hence a ValueError
+    as well as a FrontError."""
+
+
 def lib():
     global _LIB
     if _LIB is None:
@@ -53,6 +58,8 @@ def lib():
         vp = C.c_void_p
         _LIB.mvf_open_annexb.argtypes = [vp, C.c_size_t, C.POINTER(vp)]
         _LIB.mvf_open_mp4.argtypes = [vp, C.c_size_t, C.POINTER(vp)]
+        _LIB.mvf_open_ts.argtypes = [vp, C.c_size_t, C.POINTER(vp)]
+        _LIB.mvf_open_mkv.argtypes = [vp, C.c_size_t, C.POINTER(vp)]
         _LIB.mvf_close.argtypes = [vp]
         _LIB.mvf_last_error.argtypes = [vp]
         _LIB.mvf_last_error.restype = C.c_char_p
@@ -73,19 +80,21 @@ def lib():
 
 
 class Stream:
-    """An opened stream (mvf_stream): an Annex-B byte stream (mvf_open_annexb) or an MP4 / QuickTime file
-    (container="mp4", mvf_open_mp4)."""
+    """An opened stream (mvf_stream): an Annex-B byte stream (mvf_open_annexb), an MP4 / QuickTime file
+    (container="mp4", mvf_open_mp4), an MPEG-2 transport stream (container="ts", mvf_open_ts) or a Matroska / WebM
+    file (container="mkv", mvf_open_mkv)."""
 
     def __init__(self, data: bytes, container: str = "annexb"):
         self._lib = lib()
-        opener = {"annexb": self._lib.mvf_open_annexb, "mp4": self._lib.mvf_open_mp4}.get(container)
+        opener = {"annexb": self._lib.mvf_open_annexb, "mp4": self._lib.mvf_open_mp4,
+                  "ts": self._lib.mvf_open_ts, "mkv": self._lib.mvf_open_mkv}.get(container)
         if opener is None:
-            raise ValueError(f"container must be 'annexb' or 'mp4', not {container!r}")
+            raise ValueError(f"container must be 'annexb', 'mp4', 'ts' or 'mkv', not {container!r}")
         self._buf = np.frombuffer(data, np.uint8)          # keeps the bytes alive
         self.handle = C.c_void_p()
         rc = opener(self._buf.ctypes.data, len(data), C.byref(self.handle))
         if rc != 1:
-            raise FrontError(self._lib.mvf_last_error(None).decode(), rc)
+            raise OpenError(self._lib.mvf_last_error(None).decode(), rc)
         self.info = Info()
         self._lib.mvf_get_info(self.handle, C.byref(self.info))
 
